@@ -20,6 +20,9 @@ ranks of this very job and reports it as ``"parity"``.
 ``--impl reference`` times the reference's own CPU torch path (oracle/torch_path.py, the same torch calls the reference
 makes, including its python sampler) on the host cores, on a bounded sample of the same workload, and prints the same JSON
 line with "impl": "reference".
+
+``--dump-outputs DIR`` writes the losses and the parameters after the last timed step of the primary workload as
+``DIR/<name>.npy`` (float32, at most 64 MB; see ``dump_outputs``), so that two builds can be compared on the same inputs.
 """
 from __future__ import annotations
 
@@ -79,7 +82,14 @@ def parse_args():
     ap.add_argument("--no-clocks", action="store_true", help="diagnosis: do not poll nvidia-smi during the timed region")
     ap.add_argument("--cuda-graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the training step as one CUDA graph (auto: single-GPU L2-resident workloads)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the losses and parameters of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: --impl ours only")
+    return args
 
 
 def measured_peaks():
@@ -260,7 +270,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_reference_run(args.workload, args.model, max(1, min(args.steps, 2)), min(args.warmup, 1), args.gpus)
+    r = cpu_reference_run(args.workload, args.model, args.steps, args.warmup, args.gpus)
     line = {
         "impl": "reference", "metric": "epoch_s", "value": r["epoch_s"], "unit": "s", "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": r["step_ms_sample"] * r["div"], "higher_is_better": False,
@@ -484,6 +494,8 @@ def measure(job, workload, model_name, steps, warmup, cpu_steps, want_cpu, prima
         adj.phase_events = []
     total_ms, losses, launches = timed("device")
     clock_info = clocks.stop()
+    if primary and args.dump_outputs:
+        dump_outputs(args.dump_outputs, losses, model, rank, world)
     exchange = None
     if world > 1:
         # per step: propagations whose all-gather rode on the kernel epilogue (peer stores) vs NCCL collectives
@@ -569,6 +581,33 @@ def measure(job, workload, model_name, steps, warmup, cpu_steps, want_cpu, prima
     gc.collect()
     torch.cuda.empty_cache()
     return line
+
+
+DUMP_BYTES = 60 << 20  # array data of one --dump-outputs: the files stay under 64 MB with their headers
+DUMP_WHOLE_BYTES = 1 << 20  # arrays up to this size are written whole
+
+
+def dump_outputs(path, losses, model, rank, world):
+    """What the training step hands its caller after the last timed step: the losses it returns and the parameters it
+    updated, as ``path/loss.npy`` and ``path/param.<name>.npy``.  Inputs are seeded, so two builds run with the same
+    arguments can be compared file by file.  The large tables share what the small arrays leave of DUMP_BYTES and are
+    written as a fixed sample of their rows (drawn with seed 0, ascending: the same rows for the same shape).  Sharded
+    runs write every rank's owned rows as ``<name>.rank<r>.npy``."""
+    import numpy as np
+    import torch
+
+    arrays = {"loss": losses.detach()}
+    arrays.update(("param." + n, p.detach()) for n, p in model.named_parameters())
+    size = {n: t.numel() * t.element_size() for n, t in arrays.items()}
+    big = [n for n in arrays if size[n] > DUMP_WHOLE_BYTES]
+    share = (DUMP_BYTES // world - sum(s for n, s in size.items() if n not in big)) // max(len(big), 1)
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        if name in big:
+            keep = max(share // (size[name] // t.shape[0]), 1)
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(path, name + (".rank%d" % rank if world > 1 else "") + ".npy"), t.cpu().numpy())
 
 
 def spmm_roofline(workload, world, block, nnz, avg_ms, n_launch, ms_per_step, total_ms, graphed, model_name):

@@ -7,8 +7,8 @@ never does and fails loudly when ``libhgr.so`` is missing.
 Every function restates one call site of the reference (paths relative to
 ``/root/reference/HD_SELFRec``) in numpy, with the bit-sensitive inner loops in ``hgr_oracle.c``.
 Parity is PINNED: ``tests/test_oracle_golden.py`` checks every function here against
-``tests/golden/reference_vectors.npz``, produced by running the reference itself in the build
-container (``tests/golden/make_golden.py``).  The reference has no tests or golden vectors of its
+``tests/golden/reference_vectors_*.npz``, produced by running the reference itself
+(``tests/golden/make_golden.py``).  The reference has no tests or golden vectors of its
 own (SURVEY.md F3).
 
 Third-party arithmetic the reference calls on this path and that is restated here

@@ -4,7 +4,7 @@ Used (a) by tests to cross-check gradients of the CUDA path against torch autogr
 arithmetic the reference runs, and (b) by ``bench.py`` as the ``cpu_baseline`` / ``--impl reference``
 arm: the reference is pure Python over ``torch.sparse.mm`` / ``torch.mm`` / LayerNorm / Adam, and
 ``/root/reference`` does not exist on the GPU box, so the same sequence of torch calls is restated
-here (kind = "port").  Pinned against ``tests/golden/reference_vectors.npz`` by
+here (kind = "port").  Pinned against ``tests/golden/reference_vectors_*.npz`` by
 ``tests/test_oracle_golden.py::test_torch_path_*``.  Never imported by the product package.
 
 Call sites restated (paths relative to /root/reference/HD_SELFRec):

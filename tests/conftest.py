@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -13,10 +14,26 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
+class GoldenArchives(dict):
+    """The arrays of several .npz archives as one mapping, in archive order; ``files`` lists the keys like ``np.load``'s."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
 @pytest.fixture(scope="session")
 def golden():
-    """Vectors produced by the unmodified reference (tests/golden/make_golden.py)."""
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_vectors.npz"))
+    """Vectors produced by the unmodified reference (tests/golden/make_golden.py), split over
+    reference_vectors_<n>.npz so that no file exceeds 1 MB."""
+    paths = sorted(glob.glob(os.path.join(ROOT, "tests", "golden", "reference_vectors_*.npz")),
+                   key=lambda p: int(p.rsplit("_", 1)[1][:-4]))
+    assert paths, "tests/golden/reference_vectors_*.npz not found"
+    out = GoldenArchives()
+    for path in paths:
+        with np.load(path) as z:
+            out.update((k, z[k]) for k in z.files)
+    return out
 
 
 @pytest.fixture(scope="session")

@@ -15,6 +15,7 @@ stubbed.  The stubs are never on a code path whose output is stored, except
 ``torch_scatter.scatter`` for the scatter-mean form, which follows pytorch-scatter 2.1.0's
 documented semantics (sum via index_add, mean = sum / clamp(count, 1)).
 """
+import glob
 import os
 import random
 import sys
@@ -330,9 +331,22 @@ def main():
     out["eval_measures"] = np.array(measures)
     out["eval_topN"] = np.array([10, 20])
 
-    path = os.path.join(HERE, "reference_vectors.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, "(%d arrays, %.1f KB)" % (len(out), os.path.getsize(path) / 1024))
+    # consecutive runs of arrays of at most 0.9 MB go to reference_vectors_<n>.npz: float data barely compresses and no
+    # stored file may exceed 1 MB.  tests/conftest.py reads the parts back in order as one mapping
+    parts, size = [{}], 0
+    for k, a in out.items():
+        a = np.asarray(a)
+        if parts[-1] and size + a.nbytes > 900_000:
+            parts.append({})
+            size = 0
+        parts[-1][k] = a
+        size += a.nbytes
+    for old in glob.glob(os.path.join(HERE, "reference_vectors_*.npz")):
+        os.remove(old)
+    for n, part in enumerate(parts):
+        path = os.path.join(HERE, "reference_vectors_%d.npz" % n)
+        np.savez_compressed(path, **part)
+        print("wrote", path, "(%d arrays, %.1f KB)" % (len(part), os.path.getsize(path) / 1024))
 
 
 if __name__ == "__main__":

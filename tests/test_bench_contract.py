@@ -30,3 +30,30 @@ def test_other_ranks_of_the_reference_arm_exit_quietly():
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--workload", "c2",
                         "--model", "lightgcn", "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=120, env=env, cwd=ROOT)
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+def test_dump_outputs_writes_small_arrays_whole_and_a_repeatable_sample_of_large_ones(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    monkeypatch.setattr(bench, "DUMP_WHOLE_BYTES", 1 << 16)
+    model = torch.nn.Module()
+    model.emb = torch.nn.Parameter(torch.randn(20_000, 64))  # 5 MB: sampled
+    model.lin = torch.nn.Linear(64, 64)                       # 16 KB: whole
+    losses = torch.tensor([0.5, 0.25])
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), losses, model, 0, 1)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["loss.npy", "param.emb.npy", "param.lin.bias.npy", "param.lin.weight.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= (1 << 20) + 128 * len(files)
+    for f in files:
+        assert np.load(tmp_path / "a" / f).tobytes() == np.load(tmp_path / "b" / f).tobytes(), f
+    assert np.array_equal(np.load(tmp_path / "a" / "loss.npy"), losses.numpy())
+    assert np.array_equal(np.load(tmp_path / "a" / "param.lin.weight.npy"), model.lin.weight.detach().numpy())
+    emb, full = np.load(tmp_path / "a" / "param.emb.npy"), model.emb.detach().numpy()
+    assert emb.dtype == np.float32 and 1000 < emb.shape[0] < full.shape[0] and emb.shape[1] == 64
+    rows = [int(np.nonzero((full == r).all(1))[0][0]) for r in emb[:50]]
+    assert rows == sorted(rows)

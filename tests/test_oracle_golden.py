@@ -1,6 +1,6 @@
 """Pin the CPU oracle against vectors produced by the unmodified reference.
 
-The reference has no tests of its own (SURVEY.md F3); ``tests/golden/reference_vectors.npz`` holds the
+The reference has no tests of its own (SURVEY.md F3); ``tests/golden/reference_vectors_*.npz`` hold the
 outputs of the reference's classes on seeded inputs (``tests/golden/make_golden.py``).  Integer /
 index results must match exactly, floating point within the tolerance written in each test.
 """
