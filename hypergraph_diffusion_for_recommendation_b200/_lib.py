@@ -65,7 +65,6 @@ SIGNATURES = {
     "hgr_version": (C.c_int, []),
     "hgr_launch_count": (C.c_uint64, []),
     "hgr_spmm_workspace_bytes": (_SZ, [C.POINTER(CsrDesc), _I32]),
-    "hgr_set_spmm_variant": (C.c_int, [C.c_int]),
     "hgr_spmm_f32": (C.c_int, [C.POINTER(CsrDesc), _VP, _VP, _I32, C.POINTER(Epilogue), _VP, _SZ, _VP]),
     "hgr_hgconv_f32": (C.c_int, [C.POINTER(CsrDesc), C.POINTER(CsrDesc), _VP, _VP, _VP, _I32, C.POINTER(Epilogue), _VP, _SZ, _VP]),
     "hgr_lightgcn_forward_f32": (C.c_int, [C.POINTER(CsrDesc), _VP, _VP, _VP, _I32, _I32, _I32, _VP, _SZ, _VP]),

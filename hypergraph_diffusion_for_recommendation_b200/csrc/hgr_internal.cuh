@@ -59,7 +59,6 @@ __device__ __forceinline__ float4 ld_stream_f4(const float4 *p) {
                  : "l"(p));
     return v;
 }
-__device__ __forceinline__ float4 ld_ro_f4(const float4 *p) { return __ldg(p); }
 
 // One 16-byte store to a MULTICAST address: the NVSwitch delivers it to the copy of every GPU bound to the multicast object.
 __device__ __forceinline__ void st_multicast_f4(float4 *mc_addr, float4 v) {

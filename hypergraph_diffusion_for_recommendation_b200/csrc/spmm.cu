@@ -10,14 +10,13 @@
 // its nonzeros in stored order and keeps ONE accumulator chain per feature, so a row that is not
 // split is accumulated with exactly the fused multiply-add sequence of the CPU oracle
 // (oracle/hgr_oracle.c) and is bit-identical to it.  Memory-level parallelism comes from keeping
-// the gathers of the next nonzeros in flight (cp.async into a shared-memory ring, default; or a
-// batch of register loads) while the current ones are accumulated, and from prefetching the next
-// (column, value) batches -- not from splitting the sum.
+// the gathers of the next nonzeros in flight (cp.async into a shared-memory ring) while the
+// current ones are accumulated, and from prefetching the next (column, value) batches -- not from
+// splitting the sum.
 //
 // Power-law rows.  Rows longer than plan.chunk_nnz are cut into chunks of chunk_nnz nonzeros; a
 // chunk is accumulated by one group into a partial row, and a second kernel adds the partials of a
 // row in chunk order and runs the epilogue.  No atomics: results are reproducible run to run.
-// The chunk blocks are placed first in the grid because the reduce kernel waits for them.
 #include <string.h>
 
 #include "hgr_internal.cuh"
@@ -27,63 +26,18 @@ namespace hgr {
 constexpr int kThreads = 256;
 constexpr int kUnroll = 8;  // partial-row reduce kernel
 constexpr int kGroupReduceMax = 64;  // a split row with at most this many chunks is summed by one row group
+// Gather ring of 2 x kRingHalf embedding rows per thread, kMinBlocks resident blocks per SM.  Measured on B200
+// (profiles/spmm_variants_r1.md): resident warps beat deeper gather batches, staging the gathered rows through shared
+// memory with cp.async beats register loads by ~15 %, and 5 blocks leave 48 registers per thread, so the 2 x 4 ring
+// compiles without the spills it has under the 40-register cap of 6 blocks (+9 % on both shapes).
+constexpr int kRingHalf = 4;
+constexpr int kMinBlocks = 5;
+static_assert(2 * kRingHalf * kThreads * sizeof(float4) <= 48 * 1024,
+              "the gather ring must fit the 48 KB of dynamic shared memory a launch gets without cudaFuncSetAttribute");
 
-// Tuning variant (unroll depth of the gather batch x resident blocks per SM); see hgr_set_spmm_variant.
-static int g_variant = 0;  // 0 = cp.async ring of 2 x 4 rows per group, 5 blocks/SM
-
-template <int LPR, int UNR>
-__device__ __forceinline__ float4 gather_accumulate(const int32_t *__restrict__ idx, const float *__restrict__ val,
-                                                    const float4 *__restrict__ X4, int64_t s, int64_t e, int gl,
-                                                    unsigned gmask) {
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    int c = 0;
-    float v = 0.f;
-    if (s + gl < e) {
-        c = ld_stream_i32(idx + s + gl);
-        v = ld_stream_f32(val + s + gl);
-    }
-    for (int64_t base = s; base < e; base += LPR) {
-        // prefetch the next batch of (column, value) pairs while this one is consumed
-        int cn = 0;
-        float vn = 0.f;
-        const int64_t pn = base + LPR + gl;
-        if (pn < e) {
-            cn = ld_stream_i32(idx + pn);
-            vn = ld_stream_f32(val + pn);
-        }
-        const int cnt = (int)(e - base < (int64_t)LPR ? e - base : (int64_t)LPR);
-#pragma unroll
-        for (int k0 = 0; k0 < LPR; k0 += UNR) {
-            if (k0 < cnt) {
-                float4 xv[UNR];
-                float vv[UNR];
-#pragma unroll
-                for (int k = 0; k < UNR; ++k) {
-                    const int cc = __shfl_sync(gmask, c, k0 + k, LPR);
-                    vv[k] = __shfl_sync(gmask, v, k0 + k, LPR);
-                    if (k0 + k < cnt) xv[k] = ld_ro_f4(X4 + (int64_t)cc * LPR + gl);
-                }
-#pragma unroll
-                for (int k = 0; k < UNR; ++k) {
-                    if (k0 + k < cnt) {
-                        acc.x = fmaf(vv[k], xv[k].x, acc.x);
-                        acc.y = fmaf(vv[k], xv[k].y, acc.y);
-                        acc.z = fmaf(vv[k], xv[k].z, acc.z);
-                        acc.w = fmaf(vv[k], xv[k].w, acc.w);
-                    }
-                }
-            }
-        }
-        c = cn;
-        v = vn;
-    }
-    return acc;
-}
-
-// cp.async variant of the gather: every lane copies ITS 16 bytes of the next RD embedding rows straight into a
-// per-thread ring in shared memory (LDGSTS, L1 bypass) and consumes them in order, so the number of row gathers in
-// flight is bounded by shared memory (RD x 256 B per row group) instead of by what the load/store unit tracks for
-// register loads.  The accumulation order is unchanged.
+// The gather: every lane copies ITS 16 bytes of the next HB embedding rows straight into a per-thread ring in shared
+// memory (LDGSTS, L1 bypass) and consumes them in order, so the number of row gathers in flight is bounded by shared
+// memory (2 x HB rows per row group) instead of by what the load/store unit tracks for register loads.
 __device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
 }
@@ -236,11 +190,10 @@ __device__ __forceinline__ void finish_row(float4 acc, int64_t row, int gl, unsi
 }
 
 
-// What a row group works on.  Legacy layout (A.work_order == NULL): grid = [heavy chunk blocks | light row blocks] in
-// stored order.  With a work list, entry w >= 0 is a whole (unsplit) row, w < 0 is chunk ~w of the split plan; the host
-// orders the list (rows binned by length so that the two half-warps of a warp and the 16 groups of a block retire
-// together, chunk blocks interleaved with row blocks so the DRAM-bound and the L2-bound gathers overlap).  The order
-// only schedules: every row is still accumulated by ONE group in stored order, so no bit of the result depends on it.
+// What a row group works on: entry blockIdx.x * GPB + g of the work list.  Entry w >= 0 is a whole (unsplit) row, w < 0 is
+// chunk ~w of the split plan; the host orders the list (rows binned by length so that the two half-warps of a warp and the
+// 16 groups of a block retire together, items ordered by the table window they gather from so a window stays in L2).  The
+// order only schedules: every row is still accumulated by ONE group in stored order, so no bit of the result depends on it.
 struct WorkItem {
     int64_t s, e;    // nonzero range
     int64_t target;  // row (kind 0) or chunk (kind 1); -1: nothing to do
@@ -248,26 +201,16 @@ struct WorkItem {
 };
 
 template <int GPB>
-__device__ __forceinline__ WorkItem resolve_work(const hgr_csr_t &A, int g, int heavy_blocks) {
+__device__ __forceinline__ WorkItem resolve_work(const hgr_csr_t &A, int g) {
     WorkItem w;
     w.s = w.e = 0;
     w.target = -1;
     w.kind = 0;
-    int64_t chunk = -1, row = -1;
-    if (A.work_order) {
-        const int64_t wi = (int64_t)blockIdx.x * GPB + g;
-        if (wi >= A.n_work) return w;
-        const int id = A.work_order[wi];
-        if (id < 0) chunk = (int64_t)(~id);
-        else row = id;
-    } else if ((int)blockIdx.x < heavy_blocks) {
-        chunk = (int64_t)blockIdx.x * GPB + g;
-        if (chunk >= A.n_chunks) return w;
-    } else {
-        row = (int64_t)(blockIdx.x - heavy_blocks) * GPB + g;
-        if (row >= A.n_rows) return w;
-    }
-    if (chunk >= 0) {
+    const int64_t wi = (int64_t)blockIdx.x * GPB + g;
+    if (wi >= A.n_work) return w;
+    const int id = A.work_order[wi];
+    if (id < 0) {
+        const int64_t chunk = (int64_t)(~id);
         const int h = A.chunk_owner[chunk];
         const int r = A.heavy_rows[h];
         const int64_t row_end = A.indptr[r + 1];
@@ -282,40 +225,23 @@ __device__ __forceinline__ WorkItem resolve_work(const hgr_csr_t &A, int g, int 
         w.kind = 1;
         return w;
     }
-    w.s = A.indptr[row];
-    w.e = A.indptr[row + 1];
-    if (!A.work_order && A.n_heavy_rows > 0 && w.e - w.s > (int64_t)A.chunk_nnz) return w;  // summed by spmm_heavy_reduce_kernel
-    w.target = row;
+    w.s = A.indptr[id];
+    w.e = A.indptr[id + 1];
+    w.target = id;
     return w;
-}
-
-// grid = [heavy chunk blocks | light row blocks], or the blocks of A.work_order
-template <int LPR, int UNR, int MINB>
-__global__ void __launch_bounds__(kThreads, MINB) spmm_rows_kernel(hgr_csr_t A, const float4 *__restrict__ X4,
-                                                             float *__restrict__ Y, hgr_epilogue_t ep,
-                                                             float4 *__restrict__ partials, int heavy_blocks) {
-    constexpr int GPB = kThreads / LPR;
-    const int gl = threadIdx.x % LPR;
-    const int g = threadIdx.x / LPR;
-    const unsigned gmask = (LPR == 32) ? 0xffffffffu : (((1u << LPR) - 1u) << ((threadIdx.x % 32) / LPR * LPR));
-    const WorkItem w = resolve_work<GPB>(A, g, heavy_blocks);
-    if (w.target < 0) return;
-    const float4 acc = gather_accumulate<LPR, UNR>(A.indices, A.values, X4, w.s, w.e, gl, gmask);
-    if (w.kind) partials[w.target * LPR + gl] = acc;
-    else finish_row<LPR>(acc, w.target, gl, gmask, ep, Y);
 }
 
 template <int LPR, int HB, int MINB>
 __global__ void __launch_bounds__(kThreads, MINB) spmm_rows_async_kernel(hgr_csr_t A, const float4 *__restrict__ X4,
                                                                    float *__restrict__ Y, hgr_epilogue_t ep,
-                                                                   float4 *__restrict__ partials, int heavy_blocks) {
+                                                                   float4 *__restrict__ partials) {
     extern __shared__ float4 spmm_ring[];  // [2 * HB][kThreads]
     constexpr int GPB = kThreads / LPR;
     const int gl = threadIdx.x % LPR;
     const int g = threadIdx.x / LPR;
     const unsigned gmask = (LPR == 32) ? 0xffffffffu : (((1u << LPR) - 1u) << ((threadIdx.x % 32) / LPR * LPR));
     float4 *ring = spmm_ring + threadIdx.x;
-    const WorkItem w = resolve_work<GPB>(A, g, heavy_blocks);
+    const WorkItem w = resolve_work<GPB>(A, g);
     if (w.target < 0) return;
     const float4 acc = gather_accumulate_async<LPR, HB>(A.indices, A.values, X4, w.s, w.e, gl, gmask, ring);
     if (w.kind) partials[w.target * LPR + gl] = acc;
@@ -408,8 +334,7 @@ static int check_csr(const hgr_csr_t *A, const char *name) {
                 (long long)A->n_work);
     if (A->work_order)
         HGR_REQUIRE(A->n_work <= (int64_t)A->n_rows + A->n_chunks, "%s: work list longer than rows + chunks", name);
-    if (A->chunk_start)
-        HGR_REQUIRE(A->n_heavy_rows > 0 && A->work_order, "%s: explicit chunk boundaries need a split plan and a work list", name);
+    if (A->chunk_start) HGR_REQUIRE(A->n_heavy_rows > 0, "%s: explicit chunk boundaries need a split plan", name);
     return HGR_OK;
 }
 
@@ -429,75 +354,22 @@ static int check_epilogue(const hgr_epilogue_t *ep) {
     return HGR_OK;
 }
 
-template <int LPR, int UNR, int MINB>
-static int launch_spmm(const hgr_csr_t &A, const float *X, float *Y, const hgr_epilogue_t &ep, void *ws,
-                       cudaStream_t st) {
-    constexpr int GPB = kThreads / LPR;
-    const int64_t heavy_blocks = A.work_order ? 0 : (A.n_heavy_rows > 0 ? ceil_div(A.n_chunks, GPB) : 0);
-    const int64_t grid = A.work_order ? ceil_div(A.n_work, GPB) : heavy_blocks + ceil_div(A.n_rows, GPB);
-    if (grid == 0) return HGR_OK;
-    HGR_REQUIRE(grid < (int64_t)0x7fffffff, "grid too large (%lld blocks)", (long long)grid);
-    spmm_rows_kernel<LPR, UNR, MINB><<<(unsigned)grid, kThreads, 0, st>>>(A, reinterpret_cast<const float4 *>(X), Y, ep,
-                                                                          reinterpret_cast<float4 *>(ws), (int)heavy_blocks);
-    HGR_LAUNCH_OK("spmm_rows_kernel");
-    if (A.n_heavy_rows > 0) {
-        spmm_heavy_reduce_kernel<LPR><<<(unsigned)ceil_div(A.n_heavy_rows, kThreads / LPR), kThreads, 0, st>>>(
-            A, reinterpret_cast<const float4 *>(ws), Y, ep);
-        HGR_LAUNCH_OK("spmm_heavy_reduce_kernel");
-    }
-    return HGR_OK;
-}
-
-template <int LPR, int HB, int MINB>
-static int launch_spmm_async(const hgr_csr_t &A, const float *X, float *Y, const hgr_epilogue_t &ep, void *ws, cudaStream_t st) {
+template <int LPR>
+static int launch_spmm(const hgr_csr_t &A, const float *X, float *Y, const hgr_epilogue_t &ep, void *ws, cudaStream_t st) {
     constexpr int GPB = kThreads / LPR;
     float4 *partials = reinterpret_cast<float4 *>(ws);
-    const int64_t heavy_blocks = A.work_order ? 0 : (A.n_heavy_rows > 0 ? ceil_div(A.n_chunks, GPB) : 0);
-    const int64_t grid = A.work_order ? ceil_div(A.n_work, GPB) : heavy_blocks + ceil_div(A.n_rows, GPB);
+    const int64_t grid = ceil_div(A.n_work, GPB);
     if (grid == 0) return HGR_OK;
     HGR_REQUIRE(grid < (int64_t)0x7fffffff, "grid too large (%lld blocks)", (long long)grid);
-    const size_t smem = (size_t)2 * HB * kThreads * sizeof(float4);
-    {
-        // the attribute is per device: set it once for every device this process launches on
-        static std::atomic<uint64_t> done[2];  // bit d of done[d / 64]
-        int dev = 0;
-        HGR_CUDA_OK(cudaGetDevice(&dev));
-        const uint64_t bit = 1ull << (dev & 63);
-        if (dev >= 128 || !(done[(dev >> 6) & 1].load(std::memory_order_acquire) & bit)) {
-            HGR_CUDA_OK(cudaFuncSetAttribute(spmm_rows_async_kernel<LPR, HB, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            if (dev < 128) done[(dev >> 6) & 1].fetch_or(bit, std::memory_order_release);
-        }
-    }
-    spmm_rows_async_kernel<LPR, HB, MINB><<<(unsigned)grid, kThreads, smem, st>>>(A, reinterpret_cast<const float4 *>(X), Y, ep,
-                                                                                 partials, (int)heavy_blocks);
+    const size_t smem = (size_t)2 * kRingHalf * kThreads * sizeof(float4);
+    spmm_rows_async_kernel<LPR, kRingHalf, kMinBlocks><<<(unsigned)grid, kThreads, smem, st>>>(A, reinterpret_cast<const float4 *>(X), Y,
+                                                                                                ep, partials);
     HGR_LAUNCH_OK("spmm_rows_async_kernel");
     if (A.n_heavy_rows > 0) {
         spmm_heavy_reduce_kernel<LPR><<<(unsigned)ceil_div(A.n_heavy_rows, kThreads / LPR), kThreads, 0, st>>>(A, partials, Y, ep);
         HGR_LAUNCH_OK("spmm_heavy_reduce_kernel");
     }
     return HGR_OK;
-}
-
-template <int LPR>
-static int launch_spmm_variant(const hgr_csr_t &A, const float *X, float *Y, const hgr_epilogue_t &ep, void *ws,
-                               cudaStream_t st) {
-    // measured on B200 (profiles/spmm_variants_r1.md): resident warps beat deeper gather batches, and staging the
-    // gathered rows through shared memory with cp.async beats register loads by ~15 %
-    switch (g_variant) {
-        case 1: return launch_spmm<LPR, 8, 3>(A, X, Y, ep, ws, st);
-        case 2: return launch_spmm<LPR, 8, 4>(A, X, Y, ep, ws, st);
-        case 3: return launch_spmm<LPR, 4, 5>(A, X, Y, ep, ws, st);
-        case 4: return launch_spmm<LPR, 2, 8>(A, X, Y, ep, ws, st);
-        case 5: return launch_spmm<LPR, 4, 6>(A, X, Y, ep, ws, st);
-        case 6: return launch_spmm_async<LPR, 8, 3>(A, X, Y, ep, ws, st);
-        case 7: return launch_spmm_async<LPR, 2, 8>(A, X, Y, ep, ws, st);
-        case 8: return launch_spmm_async<LPR, 4, 7>(A, X, Y, ep, ws, st);
-        case 9: return launch_spmm_async<LPR, 4, 6>(A, X, Y, ep, ws, st);
-        case 10: return launch_spmm_async<LPR, 4, 4>(A, X, Y, ep, ws, st);
-        // 5 resident blocks leave 48 registers per thread: the 2 x 4 ring compiles without the spills it has under the
-        // 40-register cap of 6 blocks, +9 % on both shapes (profiles/spmm_variants_r1.md)
-        default: return launch_spmm_async<LPR, 4, 5>(A, X, Y, ep, ws, st);
-    }
 }
 
 static int spmm_impl(const hgr_csr_t *A, const float *X, float *Y, int32_t D, const hgr_epilogue_t *epi, void *ws,
@@ -513,6 +385,7 @@ static int spmm_impl(const hgr_csr_t *A, const float *X, float *Y, int32_t D, co
     if (need > 0 && (ws == nullptr || ws_bytes < need))
         return set_error(HGR_ERR_WORKSPACE, "spmm workspace: need %zu bytes, got %zu", need, ws_bytes);
     HGR_REQUIRE(aligned16(ws), "workspace must be 16-byte aligned");
+    HGR_REQUIRE(A->n_rows == 0 || A->work_order, "A: no work list (hgr_csr_t::work_order is required when n_rows > 0)");
     hgr_epilogue_t ep;
     if (epi) ep = *epi;
     else {
@@ -520,21 +393,15 @@ static int spmm_impl(const hgr_csr_t *A, const float *X, float *Y, int32_t D, co
         ep.scale = 1.f;
     }
     switch (D) {
-        case 32: return launch_spmm_variant<8>(*A, X, Y, ep, ws, st);
-        case 64: return launch_spmm_variant<16>(*A, X, Y, ep, ws, st);
-        default: return launch_spmm_variant<32>(*A, X, Y, ep, ws, st);
+        case 32: return launch_spmm<8>(*A, X, Y, ep, ws, st);
+        case 64: return launch_spmm<16>(*A, X, Y, ep, ws, st);
+        default: return launch_spmm<32>(*A, X, Y, ep, ws, st);
     }
 }
 
 }  // namespace hgr
 
 extern "C" {
-
-int hgr_set_spmm_variant(int variant) {
-    HGR_REQUIRE(variant >= 0 && variant <= 10, "variant %d out of range", variant);
-    hgr::g_variant = variant;
-    return HGR_OK;
-}
 
 size_t hgr_spmm_workspace_bytes(const hgr_csr_t *A, int32_t D) {
     if (!A || A->n_heavy_rows <= 0) return 0;

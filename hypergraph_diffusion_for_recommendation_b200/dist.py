@@ -315,12 +315,9 @@ class DistGraph:
         self.fused = (self.k is LibhgrKernels and self.world > 1 and indptr.is_cuda and self.world <= 8
                       and os.environ.get("HGR_FUSED_GATHER", "1") != "0")
         # a block whose kernel publishes its rows to many ranks spreads the whole rows through the work list, so the exchange
-        # leaves at a steady rate instead of in the first windows (graph._spread_schedule); HGR_SHARD_SCHEDULE overrides
-        sched = os.environ.get("HGR_SHARD_SCHEDULE", "auto")
-        if sched == "auto":
-            sched = "spread" if (self.fused and part.n_glob * 256 >= (1 << 30)) else ""
-        if sched and hasattr(self.block, "set_schedule"):
-            self.block.set_schedule(sched)
+        # leaves at a steady rate instead of in the first windows (graph._spread_schedule)
+        if self.fused and part.n_glob * 256 >= (1 << 30) and hasattr(self.block, "set_schedule"):
+            self.block.set_schedule("spread")
         self._pools = {}     # D -> SymmetricPool
         self._published = {}  # pool slot -> (tensor kept alive, version): local rows whose gathered copy sits in that slot
         self.publish_copy = os.environ.get("HGR_PUBLISH_COPY", "1") != "0"

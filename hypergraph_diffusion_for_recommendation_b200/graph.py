@@ -98,12 +98,6 @@ def window_split_plan(indptr: torch.Tensor, indices: torch.Tensor, window_shift:
     return heavy, ptr, owner, start
 
 
-def default_split() -> str:
-    import os
-
-    return os.environ.get("HGR_SPMM_SPLIT", "auto")
-
-
 _SPLIT_WINDOW_SHIFT = 17  # 2^17 rows = 32 MB of a D = 64 table
 _SPLIT_MIN_SEG = 128
 _SPLIT_MIN_SPAN = 3  # windows between a row's first and last column before window crossings cut it (> 64 MB of table)
@@ -115,22 +109,18 @@ _RUN = 32  # work-list entries that stay together: a whole thread block for ever
 _WINDOW_ROWS = 1 << 17  # 32 MB of a D = 64 table
 
 
-def _windowed_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, chunk_nnz, window_rows, chunk_start=None):
-    """Work items ordered by the table window their FIRST column falls in; inside a window chunks before rows, rows by
-    descending length.  Columns ascend inside a row, so the chunks of all long rows walk the gathered table front to back
-    together: a window of embedding rows is fetched from DRAM once and then served from L2 to every long row that
-    references it (popular users sit in most popular items' rows), instead of once per row."""
+def _work_items(indptr, heavy_rows, n_chunks, chunk_nnz, heavy_chunk_ptr, chunk_owner, chunk_start):
+    """What every schedule orders: the chunk entries (``~c``) with the first nonzero and length of each chunk, the non-empty whole
+    rows (ascending) with their lengths, and the empty rows (ascending)."""
     dev = indptr.device
     n_rows = indptr.numel() - 1
     deg = indptr[1:] - indptr[:-1]
-    n_chunks = int(chunk_owner.numel())
     light = torch.ones(n_rows, dtype=torch.bool, device=dev)
     if heavy_rows.numel():
         light[heavy_rows.long()] = False
     rows = torch.nonzero(light & (deg > 0)).flatten()
     empty = torch.nonzero(light & (deg == 0)).flatten()
-    r_first = indices[indptr[rows]].long() // window_rows
-    r_len = deg[rows]
+    c_ids = ~torch.arange(n_chunks, dtype=torch.int32, device=dev)
     if n_chunks:
         own = chunk_owner.long()
         row_end = indptr[heavy_rows.long()[own] + 1]
@@ -141,62 +131,54 @@ def _windowed_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner
         else:
             c_start = indptr[heavy_rows.long()[own]] + (torch.arange(n_chunks, device=dev) - heavy_chunk_ptr[own]) * chunk_nnz
             c_len = torch.clamp(row_end - c_start, max=chunk_nnz)
-        c_first = indices[c_start].long() // window_rows
     else:
-        c_first = c_len = torch.empty(0, dtype=torch.long, device=dev)
-    big = int(deg.max()) + 2 if n_rows else 2
+        c_start = c_len = torch.empty(0, dtype=torch.long, device=dev)
+    return c_ids, c_start, c_len, rows, deg[rows], empty
+
+
+def _windowed_schedule(indptr, indices, items, window_rows):
+    """Work items ordered by the table window their FIRST column falls in; inside a window chunks before rows, rows by
+    descending length.  Columns ascend inside a row, so the chunks of all long rows walk the gathered table front to back
+    together: a window of embedding rows is fetched from DRAM once and then served from L2 to every long row that
+    references it (popular users sit in most popular items' rows), instead of once per row."""
+    c_ids, c_start, c_len, rows, r_len, empty = items
+    c_first = indices[c_start].long() // window_rows
+    r_first = indices[indptr[rows]].long() // window_rows
+    big = int(indptr[-1]) + 2  # longer than any row or chunk
     # sort key: window, then descending length (a full chunk is never shorter than a whole row of the same plan, so chunks
     # lead; the groups of a block and the two half-warps of a warp get work of nearly the same length)
     key_c = c_first * (2 * big) + (big - c_len)
     key_r = r_first * (2 * big) + 1 + (big - r_len)
-    ids = torch.cat([~torch.arange(n_chunks, dtype=torch.int32, device=dev), rows.to(torch.int32)])
+    ids = torch.cat([c_ids, rows.to(torch.int32)])
     order = torch.sort(torch.cat([key_c, key_r]), stable=True).indices
     return torch.cat([ids[order], empty.to(torch.int32)]).contiguous()
 
 
-def _spread_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, chunk_nnz, window_rows, chunk_start=None):
+def _spread_schedule(indptr, indices, items, window_rows):
     """The windowed order for the chunks, with the whole rows SPREAD evenly through it instead of sitting in the window of their
     first column.  For a row-partitioned block whose propagation publishes every finished row to all ranks (fused all-gather):
     the whole rows are most of the output rows, and in the windowed order they all run in the first windows (every user row starts
     in rank 0's item range), so the exchange is squeezed into the first half of the kernel and stalls it.  Here runs of ``_RUN``
     rows of equal length (a whole thread block) are shuffled with a fixed seed and merged with the chunk runs in proportion to
     their nonzeros: finished rows -- and the NVLink traffic they cause -- leave at a steady rate from the first block to the last."""
+    c_ids, c_start, c_len, rows, r_len, empty = items
+    if c_ids.numel() == 0 or rows.numel() == 0:
+        return _windowed_schedule(indptr, indices, items, window_rows)
     dev = indptr.device
-    n_rows = indptr.numel() - 1
-    deg = indptr[1:] - indptr[:-1]
-    n_chunks = int(chunk_owner.numel())
-    light = torch.ones(n_rows, dtype=torch.bool, device=dev)
-    if heavy_rows.numel():
-        light[heavy_rows.long()] = False
-    rows = torch.nonzero(light & (deg > 0)).flatten()
-    empty = torch.nonzero(light & (deg == 0)).flatten()
-    if n_chunks == 0 or rows.numel() == 0:
-        return _windowed_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, chunk_nnz, window_rows, chunk_start)
     # chunks: window of the first column, then descending length
-    own = chunk_owner.long()
-    row_end = indptr[heavy_rows.long()[own] + 1]
-    if chunk_start is not None:
-        c_start = chunk_start
-        last = torch.arange(1, n_chunks + 1, device=dev) == heavy_chunk_ptr[own + 1]
-        c_len = torch.where(last, row_end, torch.cat([chunk_start[1:], chunk_start[:1]])) - c_start
-    else:
-        c_start = indptr[heavy_rows.long()[own]] + (torch.arange(n_chunks, device=dev) - heavy_chunk_ptr[own]) * chunk_nnz
-        c_len = torch.clamp(row_end - c_start, max=chunk_nnz)
-    big = int(deg.max()) + 2
+    big = int(indptr[-1]) + 2  # longer than any chunk
     c_order = torch.sort((indices[c_start].long() // window_rows) * big + (big - c_len), stable=True).indices
-    c_ids = (~torch.arange(n_chunks, dtype=torch.int32, device=dev))[c_order]
-    c_len = c_len[c_order]
+    c_ids, c_len = c_ids[c_order], c_len[c_order]
     # rows: runs of equal length, shuffled
-    r_order = torch.sort(deg[rows], descending=True, stable=True).indices
-    rows = rows[r_order]
+    r_order = torch.sort(r_len, descending=True, stable=True).indices
     n_runs = -(-int(rows.numel()) // _RUN)
     gen = torch.Generator()
     gen.manual_seed(0x5eed)
     run_pos = torch.empty(n_runs, dtype=torch.long)
     run_pos[torch.randperm(n_runs, generator=gen)] = torch.arange(n_runs)
     slot = run_pos.to(dev)[torch.arange(rows.numel(), device=dev) // _RUN] * _RUN + torch.arange(rows.numel(), device=dev) % _RUN
-    rows = rows[torch.sort(slot).indices]
-    r_len = deg[rows]
+    r_order = r_order[torch.sort(slot).indices]
+    rows, r_len = rows[r_order], r_len[r_order]
 
     def run_keys(lengths):  # fraction of the list's nonzeros that precede the run an entry belongs to
         n = lengths.numel()
@@ -210,76 +192,40 @@ def _spread_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, 
 
 def work_schedule(indptr: torch.Tensor, heavy_rows: torch.Tensor, n_chunks: int, chunk_nnz: int, mode: str,
                   indices: torch.Tensor | None = None, heavy_chunk_ptr: torch.Tensor | None = None,
-                  chunk_owner: torch.Tensor | None = None, n_cols: int = 0, chunk_start: torch.Tensor | None = None) -> torch.Tensor | None:
+                  chunk_owner: torch.Tensor | None = None, n_cols: int = 0, chunk_start: torch.Tensor | None = None) -> torch.Tensor:
     """The ``hgr_csr_t::work_order`` list (int32, device): which row or chunk every row group of the propagation kernel takes.
 
     ``binned``       chunk entries first, then the unsplit rows by descending length (stable): the two half-warps of a
                      warp and the groups of a block get rows of (nearly) the same length and retire together, and the
                      longest rows start first, so the grid has no long-row tail.
-    ``interleaved``  the same two lists merged run by run (``_RUN`` entries) in proportion to their nonzeros: chunks
-                     (mostly popular items gathering from the large user table: DRAM-bound) and rows (mostly users
-                     gathering from the L2-resident item table) are in flight together instead of one after the other.
     ``windowed[:W]`` items ordered by the W-row window of the gathered table their first column falls in (``_windowed_schedule``).
     ``spread[:W]``   the windowed order for the chunks, whole rows spread evenly through it (``_spread_schedule``): the schedule of a
                      row-partitioned block whose kernel publishes its rows to many ranks.
     ``auto``         ``windowed`` when the gathered table is larger than 64 MB, else ``binned`` (the default).
-    ``stored``       no list (rows in stored order, chunk blocks first).
 
-    Measured on B200 (profiles/spmm_r2.md), 1.25 M x 0.25 M x 125 M graph, one launch: stored 6.27 ms, binned 4.71 - 5.01,
-    interleaved 5.29 (worse than binned: the two gather streams evict each other from L2), windowed 4.13 - 4.20.
+    Measured on B200 (profiles/spmm_r2.md), 1.25 M x 0.25 M x 125 M graph, one launch: rows in stored order without a list
+    6.27 ms, binned 4.71 - 5.01, windowed 4.13 - 4.20.
     Only the schedule changes: each row is accumulated by one row group in stored order, so results are bit-identical."""
     if mode == "auto":
         # a table that fits L2 (<= 64 MB of 256-byte rows) needs no windows: pure length binning measured 10 % faster there
         mode = "windowed" if n_cols * 256 > (64 << 20) else "binned"
-    if mode == "stored":
-        return None
-    if mode.startswith("spread"):
-        return _spread_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, chunk_nnz,
-                                int(mode.split(":")[1]) if ":" in mode else _WINDOW_ROWS, chunk_start)
-    if mode.startswith("windowed"):
-        return _windowed_schedule(indptr, indices, heavy_rows, heavy_chunk_ptr, chunk_owner, chunk_nnz,
-                                  int(mode.split(":")[1]) if ":" in mode else _WINDOW_ROWS, chunk_start)
-    if mode not in ("binned", "interleaved"):
-        raise ValueError("unknown propagation schedule %r" % (mode,))
-    n_rows = indptr.numel() - 1
-    if n_rows == 0:
-        return None
-    dev = indptr.device
-    deg = indptr[1:] - indptr[:-1]
-    light = torch.ones(n_rows, dtype=torch.bool, device=dev)
-    if heavy_rows.numel():
-        light[heavy_rows.long()] = False
-    rows = torch.nonzero(light).flatten()
-    ldeg = deg[rows]
-    order = torch.sort(ldeg, descending=True, stable=True).indices
-    rows, ldeg = rows[order].to(torch.int32), ldeg[order]
-    chunks = ~torch.arange(n_chunks, dtype=torch.int32, device=dev)
-    if mode == "binned" or n_chunks == 0 or rows.numel() == 0:
-        return torch.cat([chunks, rows]).contiguous()
-    # position of every run in its own list, as the fraction of the list's nonzeros that precede it
-    run_l = torch.arange(rows.numel(), device=dev) // _RUN
-    before = torch.cumsum(ldeg, 0) - ldeg
-    first = before[torch.arange(0, rows.numel(), _RUN, device=dev)]
-    key_l = first.to(torch.float64)[run_l] / max(float(ldeg.sum()), 1.0)
-    run_c = torch.arange(n_chunks, device=dev) // _RUN
-    key_c = (run_c * _RUN).to(torch.float64) / float(n_chunks)
-    keys = torch.cat([key_c, key_l])
-    merged = torch.sort(keys, stable=True).indices  # ties: the chunk run first
-    return torch.cat([chunks, rows])[merged].contiguous()
-
-
-def default_schedule() -> str:
-    import os
-
-    return os.environ.get("HGR_SPMM_SCHEDULE", "auto")
+    name, _, window = mode.partition(":")
+    if name not in ("binned", "windowed", "spread") or (name == "binned" and window):
+        raise ValueError("unknown propagation schedule %r (auto | binned | windowed[:W] | spread[:W])" % (mode,))
+    items = _work_items(indptr, heavy_rows, n_chunks, chunk_nnz, heavy_chunk_ptr, chunk_owner, chunk_start)
+    if name == "binned":
+        c_ids, _, _, rows, r_len, empty = items
+        order = torch.sort(r_len, descending=True, stable=True).indices
+        return torch.cat([c_ids, rows[order].to(torch.int32), empty.to(torch.int32)]).contiguous()
+    schedule = _spread_schedule if name == "spread" else _windowed_schedule
+    return schedule(indptr, indices, items, int(window) if window else _WINDOW_ROWS)
 
 
 class DeviceCSR:
     """CSR matrix in device memory + split plan + work schedule + ctypes descriptor (``hgr_csr_t``)."""
 
     def __init__(self, indptr: torch.Tensor, indices: torch.Tensor, values: torch.Tensor, shape, symmetric: bool = False,
-                 chunk_nnz: int | None = None, transpose: "DeviceCSR | None" = None, schedule: str | None = None,
-                 split: str | None = None):
+                 chunk_nnz: int | None = None, transpose: "DeviceCSR | None" = None, split: str = "auto"):
         if indptr.dtype != torch.int64 or indices.dtype != torch.int32 or values.dtype != torch.float32:
             raise TypeError("DeviceCSR wants int64 indptr, int32 indices, float32 values")
         if not (indptr.is_cuda and indices.is_cuda and values.is_cuda):
@@ -295,7 +241,6 @@ class DeviceCSR:
         # How long rows are cut.  "fixed": every chunk_nnz nonzeros.  "window[:shift[:min_seg[:min_span]]]": where the row leaves a window of
         # 2^shift rows of the gathered table (window_split_plan), at most chunk_nnz nonzeros per chunk.  "auto": windows when the
         # gathered table cannot stay in L2 (> 64 MB of 256-byte rows) and the caller did not fix chunk_nnz, else fixed.
-        split = split or default_split()
         if split == "auto":
             split = "window" if (self.shape[1] * 256 > (64 << 20) and not chunk_nnz and nnz > 0) else "fixed"
         self.split = split
@@ -323,18 +268,16 @@ class DeviceCSR:
                                                           self.chunk_owner.data_ptr())
         d.chunk_start = None if self.chunk_start is None or d.n_chunks == 0 else self.chunk_start.data_ptr()
         self.desc = d
-        self.set_schedule(schedule or default_schedule())
+        self.set_schedule("auto")
 
     def set_schedule(self, mode: str) -> "DeviceCSR":
         """Choose how the propagation kernel's row groups are handed rows and chunks (``work_schedule``); results do not change."""
-        if mode == "stored" and self.desc.chunk_start:
-            mode = "binned"  # chunks with explicit boundaries are only reachable through a work list
         self.schedule = mode
         self.work_order = work_schedule(self.indptr, self.heavy_rows, int(self.desc.n_chunks), self.chunk_nnz, mode, self.indices,
                                         self.heavy_chunk_ptr, self.chunk_owner, self.shape[1],
                                         self.chunk_start if self.desc.chunk_start else None)
-        self.desc.work_order = None if self.work_order is None else self.work_order.data_ptr()
-        self.desc.n_work = 0 if self.work_order is None else int(self.work_order.numel())
+        self.desc.work_order = self.work_order.data_ptr()
+        self.desc.n_work = int(self.work_order.numel())
         return self
 
     # ---- what the reference's encoders touch on the sparse tensor -------------------------------

@@ -66,12 +66,12 @@ typedef struct {
     const int32_t *heavy_rows;      /* [n_heavy_rows] */
     const int64_t *heavy_chunk_ptr; /* [n_heavy_rows + 1] */
     const int32_t *chunk_owner;     /* [n_chunks] */
-    /* Optional schedule of the propagation kernel: entry w >= 0 is unsplit row w, entry w < 0 is chunk ~w of the
-     * split plan; 16 consecutive entries (D = 64) share a thread block.  Every unsplit row and every chunk must
-     * appear exactly once.  graph.py bins rows by length and interleaves chunk blocks with row blocks; the order
-     * never changes a result bit (each row is still accumulated by one row group in stored order).
-     * NULL: rows in stored order, chunk blocks first. */
-    const int32_t *work_order; /* [n_work] or NULL */
+    /* Schedule of the propagation kernel, required whenever n_rows > 0: entry w >= 0 is unsplit row w, entry
+     * w < 0 is chunk ~w of the split plan; 16 consecutive entries (D = 64) share a thread block.  Every unsplit
+     * row and every chunk must appear exactly once.  graph.py bins rows by length or orders them by the window
+     * of the gathered table they read; the order never changes a result bit (each row is still accumulated by
+     * one row group in stored order). */
+    const int32_t *work_order; /* [n_work] */
     int64_t n_work;
     const int64_t *chunk_start; /* [n_chunks] first nonzero of every chunk, or NULL: chunk k of a row starts at k * chunk_nnz */
 } hgr_csr_t;
@@ -130,10 +130,6 @@ int hgr_window_split_count(const int64_t *indptr, const int32_t *indices, int32_
 int hgr_window_split_fill(const int64_t *indptr, const int32_t *indices, const int32_t *heavy_rows, const int64_t *heavy_chunk_ptr,
                           int32_t n_heavy_rows, int32_t window_shift, int32_t min_seg, int32_t max_seg, int32_t min_span, int64_t *chunk_start,
                           hgr_stream_t stream);
-/* Tuning hook of the propagation kernel (gather depth x resident blocks per SM).  0 [default], 6, 7, 8, 9, 10: embedding
- * rows staged through a shared-memory ring with cp.async (2x4 x 5, 2x8 x 3, 2x2 x 8, 2x4 x 7, 2x4 x 6, 2x4 x 4); 1-5: register gathers
- * (8 x 3, 8 x 4, 4 x 5, 2 x 8, 4 x 6).  Results do not depend on it. */
-int hgr_set_spmm_variant(int variant);
 int hgr_spmm_f32(const hgr_csr_t *A, const float *X, float *Y, int32_t D, const hgr_epilogue_t *epi,
                  void *workspace, size_t workspace_bytes, hgr_stream_t stream);
 

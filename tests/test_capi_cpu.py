@@ -141,8 +141,8 @@ def test_shape_predicates_refuse_cpu_tensors_and_odd_widths():
         ops.hyperedge(torch.ones(8, 128), torch.ones(8, 64))
 
 
-@pytest.mark.parametrize("mode", ["binned", "interleaved", "windowed", "windowed:7", "spread", "spread:7", "auto"])
-def test_work_schedule_lists_every_row_and_chunk_once(mode):
+@pytest.mark.parametrize("mode", ["binned", "windowed", "windowed:7", "windowed:1", "spread", "spread:7", "spread:1", "auto"])
+def test_work_list_names_every_row_and_chunk_once(mode):
     """hgr_csr_t::work_order: whatever the order, each unsplit row and each chunk of the split plan appears exactly once."""
     import numpy as np
     import torch
@@ -168,7 +168,20 @@ def test_work_schedule_lists_every_row_and_chunk_once(mode):
     if mode == "binned":  # chunks first, then rows by descending length
         r = order[order >= 0]
         assert (order[: owner.size] < 0).all() and (np.diff(deg[r]) <= 0).all()
-    assert graph.work_schedule(torch.from_numpy(indptr), torch.from_numpy(heavy), int(owner.size), chunk, "stored") is None
+
+
+@pytest.mark.parametrize("mode", ["stored", "interleaved", "binned:7", "window", "spread7"])
+def test_work_schedule_refuses_unknown_modes(mode):
+    """Every row group takes its work from the list, so there is no list-free ``stored`` order; ``interleaved`` was measured
+    slower than ``binned`` and is gone too.  Neither they nor a malformed mode silently fall back to another schedule."""
+    import torch
+
+    from hypergraph_diffusion_for_recommendation_b200 import graph
+
+    indptr = torch.tensor([0, 2, 2, 5], dtype=torch.int64)
+    with pytest.raises(ValueError):
+        graph.work_schedule(indptr, torch.zeros(0, dtype=torch.int32), 0, 64, mode, torch.tensor([0, 1, 0, 1, 2], dtype=torch.int32),
+                            torch.zeros(1, dtype=torch.int64), torch.zeros(0, dtype=torch.int32), 3)
 
 
 def test_window_split_plan_rule():

@@ -96,6 +96,26 @@ def test_spmm_empty_rows_and_empty_matrix(hgr):
         hgr.ops.spmm_raw(a, torch.ones(5, 64))  # CPU tensor: no fallback
 
 
+def test_spmm_refuses_a_matrix_without_work_list(hgr, pl_graph):
+    """Row groups take their rows and chunks from hgr_csr_t::work_order only: the descriptor of a non-empty matrix without a
+    list is refused before anything is launched.  Every pointer is valid device memory, so a library that accepted the
+    descriptor would run the product instead of failing."""
+    import ctypes as C
+
+    n = pl_graph["n_users"] + pl_graph["n_items"]
+    a = hgr.graph.DeviceCSR.from_host(*pl_graph["csr"], (n, n), symmetric=True, split="fixed")
+    d = hgr.lib.CsrDesc.from_buffer_copy(a.desc)
+    d.work_order, d.n_work = None, 0
+    x, y = torch.ones(n, 64, device="cuda"), torch.zeros(n, 64, device="cuda")
+    ws = a.workspace(64)
+    lib = hgr.lib.lib()
+    before = lib.hgr_launch_count()
+    rc = lib.hgr_spmm_f32(C.byref(d), x.data_ptr(), y.data_ptr(), 64, None, hgr.lib.ptr(ws), 0 if ws is None else ws.numel() * 4,
+                          hgr.lib.stream_ptr())
+    assert rc == -1 and b"work list" in lib.hgr_last_error()
+    assert lib.hgr_launch_count() == before
+
+
 def test_spmm_epilogue_stages(hgr, pl_graph, adj):
     n = pl_graph["n_users"] + pl_graph["n_items"]
     rng = np.random.default_rng(3)
@@ -511,7 +531,7 @@ def test_drop_edges_philox_mask_is_a_consistent_transpose_pair_and_changes_with_
     assert rel_err(x.grad, want) < RTOL
 
 
-def test_window_split_plan_device_matches_rule_and_oracle(hgr, pl_graph):
+def test_window_split_plan_matches_rule_and_oracle_under_every_schedule(hgr, pl_graph):
     """The window-aligned split plan (csrc/split_plan.cu): the device walk gives the plan of the python restatement; the
     propagation with it is reproducible, independent of the schedule, within 1e-5 of the oracle and bit-exact on whole rows."""
     from hypergraph_diffusion_for_recommendation_b200 import graph
@@ -531,7 +551,7 @@ def test_window_split_plan_device_matches_rule_and_oracle(hgr, pl_graph):
     x = np.random.default_rng(3).standard_normal((n, 64)).astype(np.float32)
     ref = O.spmm(indptr, indices, vals, x)
     outs = []
-    for sched in ("binned", "windowed:16", "interleaved", "stored"):
+    for sched in ("binned", "windowed:16", "spread:16"):
         a.set_schedule(sched)
         outs.append(hgr.ops.spmm_raw(a, cuda(x)))
     for y in outs[1:]:

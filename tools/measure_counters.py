@@ -2,7 +2,7 @@
 
     python tools/measure_counters.py [--what spmm_c5w,spmm_c5w8,spmm_c4,eval_c5w,eval_c4] [--out gpurun_out/kernel_counters.json]
 
-Runs `ncu --metrics ... --clock-control none -k regex:<kernel> -c <n>` over the probe scripts (one GPU; never a bench number)
+Runs `ncu --metrics ... --clock-control none -k regex:<kernel> --launch-skip <s> -c <n>` over the probe scripts (one GPU; never a bench number)
 and writes, keyed the way bench.py looks them up (`profiles/kernel_counters.json` after the file is copied there):
 
   spmm:<workload>:<world>:<schedule>   (schedule = what DeviceCSR.schedule reports: auto, or spread for the blocks of >= 4 ranks) dram_read_bytes, dram_write_bytes, l2_to_sm_bytes, l2_hit_pct, duration_ms
@@ -25,16 +25,17 @@ EVAL_METRICS = ("sm__pipe_tensor_cycles_active.avg.pct_of_peak_sustained_elapsed
                 "sm__cycles_active.avg,sm__cycles_elapsed.max,gpu__time_duration.sum")
 
 JOBS = {
-    # name: (cache key prefix, kernel regex, launches to capture, probe command)
-    "spmm_c5w": ("spmm:c5w:1", "spmm_rows_async", 1, ["tools/spmm_probe.py", "--shapes", "1250000x250000x125000000", "--variants", "0", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
-    "spmm_c5w8": ("spmm:c5w:8", "spmm_rows_async", 1, ["tools/shard_probe.py", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
-    "spmm_c5w4": ("spmm:c5w:4", "spmm_rows_async", 1, ["tools/shard_probe.py", "--world", "4", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
-    "spmm_c5w2": ("spmm:c5w:2", "spmm_rows_async", 1, ["tools/shard_probe.py", "--world", "2", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
-    "spmm_c5w8s": ("spmm:c5w:8", "spmm_rows_async", 1, ["tools/shard_probe.py", "--schedules", "spread", "--splits", "auto", "--iters", "1"]),
-    "spmm_c5w4s": ("spmm:c5w:4", "spmm_rows_async", 1, ["tools/shard_probe.py", "--world", "4", "--schedules", "spread", "--splits", "auto", "--iters", "1"]),
-    "spmm_c4": ("spmm:c4:1", "spmm_rows_async", 1, ["tools/spmm_probe.py", "--shapes", "52000x92000x3000000", "--variants", "0", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
-    "eval_c5w": ("eval:c5w:1", "eval_scores", 2, ["tools/eval_probe.py", "--shape", "c5e", "--users", "262144", "--iters", "1"]),
-    "eval_c4": ("eval:c4:1", "eval_scores", 2, ["tools/eval_probe.py", "--shape", "c4", "--iters", "1"]),
+    # name: (cache key prefix, kernel regex, matching launches to skip, launches to capture, probe command)
+    # spmm_probe.py first runs two reference propagations (no split plan, then the binned schedule): skipped.
+    "spmm_c5w": ("spmm:c5w:1", "spmm_rows_async", 2, 1, ["tools/spmm_probe.py", "--shapes", "1250000x250000x125000000", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
+    "spmm_c5w8": ("spmm:c5w:8", "spmm_rows_async", 0, 1, ["tools/shard_probe.py", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
+    "spmm_c5w4": ("spmm:c5w:4", "spmm_rows_async", 0, 1, ["tools/shard_probe.py", "--world", "4", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
+    "spmm_c5w2": ("spmm:c5w:2", "spmm_rows_async", 0, 1, ["tools/shard_probe.py", "--world", "2", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
+    "spmm_c5w8s": ("spmm:c5w:8", "spmm_rows_async", 0, 1, ["tools/shard_probe.py", "--schedules", "spread", "--splits", "auto", "--iters", "1"]),
+    "spmm_c5w4s": ("spmm:c5w:4", "spmm_rows_async", 0, 1, ["tools/shard_probe.py", "--world", "4", "--schedules", "spread", "--splits", "auto", "--iters", "1"]),
+    "spmm_c4": ("spmm:c4:1", "spmm_rows_async", 2, 1, ["tools/spmm_probe.py", "--shapes", "52000x92000x3000000", "--schedules", "auto", "--splits", "auto", "--iters", "1"]),
+    "eval_c5w": ("eval:c5w:1", "eval_scores", 0, 2, ["tools/eval_probe.py", "--shape", "c5e", "--users", "262144", "--iters", "1"]),
+    "eval_c4": ("eval:c4:1", "eval_scores", 0, 2, ["tools/eval_probe.py", "--shape", "c4", "--iters", "1"]),
 }
 
 
@@ -44,10 +45,10 @@ def to_number(value, unit):
     return v * scale.get(unit, 1.0)
 
 
-def run_ncu(regex, count, metrics, cmd):
+def run_ncu(regex, skip, count, metrics, cmd):
     log = tempfile.NamedTemporaryFile(suffix=".csv", delete=False).name
-    full = ["ncu", "--metrics", metrics, "--clock-control", "none", "-k", "regex:" + regex, "-c", str(count), "--csv", "--log-file", log,
-            sys.executable] + cmd
+    full = ["ncu", "--metrics", metrics, "--clock-control", "none", "-k", "regex:" + regex, "--launch-skip", str(skip), "-c", str(count),
+            "--csv", "--log-file", log, sys.executable] + cmd
     subprocess.run(full, cwd=ROOT, check=True, stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     rows = list(csv.reader(open(log, errors="replace")))
     hdr = next(k for k, r in enumerate(rows) if r and r[0] == "ID")
@@ -72,8 +73,8 @@ def main():
         if path and os.path.exists(path):
             out.update(json.load(open(path)))
     for name in args.what.split(","):
-        prefix, regex, count, cmd = JOBS[name]
-        launches = run_ncu(regex, count, SPMM_METRICS if prefix.startswith("spmm") else EVAL_METRICS, cmd)
+        prefix, regex, skip, count, cmd = JOBS[name]
+        launches = run_ncu(regex, skip, count, SPMM_METRICS if prefix.startswith("spmm") else EVAL_METRICS, cmd)
         src = "ncu --metrics (tools/measure_counters.py %s): %s" % (name, " ".join(cmd))
         if prefix.startswith("spmm"):
             (_, kname), m = next(iter(launches.items()))

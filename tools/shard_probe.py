@@ -23,8 +23,7 @@ def main():
     ap.add_argument("--world", type=int, default=8)
     ap.add_argument("--rank", type=int, default=0)
     ap.add_argument("--iters", type=int, default=5)
-    ap.add_argument("--variants", default="0", help="hgr_set_spmm_variant values to time (include/hgr.h)")
-    ap.add_argument("--schedules", default="stored,binned,windowed", help="work schedules to time (graph.work_schedule)")
+    ap.add_argument("--schedules", default="binned,windowed,spread", help="work schedules to time (graph.work_schedule)")
     ap.add_argument("--splits", default="fixed", help="split plans: fixed | window[:shift[:min_seg]]")
     ap.add_argument("--chunks", default="0", help="chunk_nnz values of the split plan to time (0 = the default rule)")
     args = ap.parse_args()
@@ -41,8 +40,6 @@ def main():
     print("block %d of %d: rows %d cols %d nnz %d, heavy rows %d, built in %.1f s" % (
         args.rank, args.world, part.n_loc, part.n_glob, block._nnz(), block.desc.n_heavy_rows, time.time() - t0), flush=True)
     x = torch.randn(part.n_glob, 64, device=dev)
-    from hypergraph_diffusion_for_recommendation_b200 import _lib
-
     deg = (indptr[1:] - indptr[:-1])
     for name, dsel in (("user rows", deg[:part.up]), ("item rows", deg[part.up:])):
         tot = int(dsel.sum())
@@ -53,8 +50,8 @@ def main():
         print("  " + " | ".join(line), flush=True)
     del block
     made = None
-    for chunk, split, sched, variant in ((int(c), sp, s, int(v)) for c in args.chunks.split(",") for sp in args.splits.split(",")
-                                         for s in args.schedules.split(",") for v in args.variants.split(",")):
+    for chunk, split, sched in ((int(c), sp, s) for c in args.chunks.split(",") for sp in args.splits.split(",")
+                                for s in args.schedules.split(",")):
         if made != (chunk, split):
             block = None
             torch.cuda.empty_cache()
@@ -65,8 +62,7 @@ def main():
             print("split %s chunk_nnz %d: heavy rows %d, chunks %d, plan %.2f s" % (block.split, block.chunk_nnz, block.desc.n_heavy_rows,
                                                                                block.desc.n_chunks, time.time() - t0), flush=True)
         block.set_schedule(sched)
-        _lib.check(_lib.lib().hgr_set_spmm_variant(variant))
-        print("schedule %s variant %d" % (sched, variant), flush=True)
+        print("schedule %s" % sched, flush=True)
         for _ in range(2):
             y = ops.spmm_raw(block, x)
         ts = []

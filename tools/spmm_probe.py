@@ -7,7 +7,7 @@ import time
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from hypergraph_diffusion_for_recommendation_b200 import _lib, ops  # noqa: E402
+from hypergraph_diffusion_for_recommendation_b200 import ops  # noqa: E402
 from hypergraph_diffusion_for_recommendation_b200.synth import norm_adj_from_pairs_torch, powerlaw_interactions_device  # noqa: E402
 
 
@@ -20,8 +20,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--shapes", default="52000x92000x3000000,1250000x250000x125000000")
     ap.add_argument("--chunks", default="0")
-    ap.add_argument("--variants", default="0")
-    ap.add_argument("--schedules", default="stored,binned,interleaved")
+    ap.add_argument("--schedules", default="binned,windowed")
     ap.add_argument("--splits", default="fixed", help="split plans to time: fixed | window[:shift[:min_seg]] (graph.DeviceCSR)")
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--d", type=int, default=64)
@@ -38,7 +37,6 @@ def main():
         base = norm_adj_from_pairs_torch(u, i, U, I, chunk_nnz=1 << 30)
         n, nnz = U + I, base._nnz()
         x = torch.randn(n, args.d, device=dev)
-        _lib.check(_lib.lib().hgr_set_spmm_variant(5))  # register-gather kernel: keeps `ncu -k spmm_rows_async -c 1` on the timed launches
         y_seq = ops.spmm_raw(base, x).clone()  # every row accumulated sequentially (no split plan)
         for chunk, split in ((int(c), sp) for c in args.chunks.split(",") for sp in args.splits.split(",")):
             torch.cuda.synchronize()
@@ -49,18 +47,16 @@ def main():
             deg = adj.indptr[1:] - adj.indptr[:-1]
             print("shape %s nnz %d plan %.2fs split %s chunk %d heavy_rows %d chunks %d maxdeg %d" % (
                 shape, nnz, t2 - t1, adj.split, adj.chunk_nnz, adj.desc.n_heavy_rows, adj.desc.n_chunks, int(deg.max())), flush=True)
-            _lib.check(_lib.lib().hgr_set_spmm_variant(5))
             adj.set_schedule("binned")
             y_ref = ops.spmm_raw(adj, x).clone()
             err = ((y_ref - y_seq).abs().amax(1) / y_seq.abs().amax(1).clamp(min=1e-30)).max()
             print("  vs sequential rows: worst row-wise relative difference %.2e" % float(err), flush=True)
-            for sched, variant in ((s, int(v)) for s in args.schedules.split(",") for v in args.variants.split(",")):
+            for sched in args.schedules.split(","):
                 adj.set_schedule(sched)
-                _lib.check(_lib.lib().hgr_set_spmm_variant(variant))
                 for _ in range(3):
                     y = ops.spmm_raw(adj, x)
                 if not torch.equal(y, y_ref):
-                    print("  variant %d: RESULT DIFFERS from the static kernel (max abs %.3e)" % (variant, float((y - y_ref).abs().max())))
+                    print("  %s: RESULT DIFFERS from the binned schedule (max abs %.3e)" % (sched, float((y - y_ref).abs().max())))
                 times = []
                 for _ in range(args.iters):
                     flush.fill_(1)
@@ -72,8 +68,8 @@ def main():
                     times.append(s.elapsed_time(e))
                 ms = sorted(times)[len(times) // 2]
                 b = algorithmic_bytes(n, nnz, args.d)
-                print("  %-11s variant %d | spmm median %.3f ms min %.3f ms | alg %.1f MB -> %.0f GB/s | %.1f Gnnz/s" % (
-                    sched, variant, ms, min(times), b / 1e6, b / ms / 1e6, nnz / ms / 1e6), flush=True)
+                print("  %-11s | spmm median %.3f ms min %.3f ms | alg %.1f MB -> %.0f GB/s | %.1f Gnnz/s" % (
+                    sched, ms, min(times), b / 1e6, b / ms / 1e6, nnz / ms / 1e6), flush=True)
             del adj, y
         del base, x, y_seq
 
