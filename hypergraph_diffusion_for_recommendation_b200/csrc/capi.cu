@@ -20,7 +20,7 @@ extern "C" {
 
 const char *hgr_last_error(void) { return hgr::t_error; }
 
-int hgr_version(void) { return 101; }  // 0.1.1
+int hgr_version(void) { return 102; }  // 0.1.2
 
 uint64_t hgr_launch_count(void) { return hgr::g_launches.load(std::memory_order_relaxed); }
 

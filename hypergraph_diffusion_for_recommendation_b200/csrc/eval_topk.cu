@@ -21,15 +21,19 @@
 //        eval_tau_kernel     K-th largest bucket maximum = a lower bound tau of the user's K-th best score.
 //        FILTER pass         over all item tiles: scores >= tau - 2 eps are appended to the user's candidate
 //                            list.  Scores never leave the SM; only ~(4 K + window) (score, id) pairs per user do.
+//                            Long lists (64 < K <= 256): one pool of up to 8 K slots per user, filled through a
+//                            per-user append counter, instead of one short list per (sub-range, column half, user).
 //   3. eval_rescore_kernel   approximate K-th best among the candidates prunes the list, the survivors are
 //                            re-scored exactly in fp32 in the canonical order (ascending-k fused multiply-add,
 //                            oracle/hgr_oracle.c hgr_oracle_scores_f32), exact top-K: score descending, ties by
 //                            ascending item id.  |bf16 score - fp32 score| <= eps(user) is a proven bound, so
 //                            the candidate set is a superset of the true top-K: bit-identical to the oracle.
+//                            Long lists: one block per user sorts its pool in shared memory instead.
 //   4. eval_brute_kernel     exact SIMT fallback for users whose candidate list overflowed (and the whole
-//                            job when D != 64 or K > 64): every score in fp32, K rounds of block arg-max.
+//                            job when D != 64 or K > 256): every score in fp32, K rounds of block arg-max.
 //   5. eval_refquirk_kernel  optional: replays find_k_largest's re-visit of the first K candidates
 //                            (SURVEY.md F9) so that Recall/NDCG strings match the reference bit for bit.
+//                            One warp per user for K <= 64, one block per user for long lists.
 #include <cuda_bf16.h>
 #include <math_constants.h>
 #include <string.h>
@@ -54,6 +58,9 @@ constexpr int EV_TMEM_COLS = 512;
 constexpr int EV_SAMPLE_STRIDE = 4;                 // the sample pass scores 1 / 4 of the item tiles
 constexpr int EV_BUCKETS = 32;                      // bucket maxima per (user, sample segment)
 constexpr float EV_MASK_SCORE = -10e8f;             // base/graph_recommender.py:80
+constexpr int EV_LIST_K = 64;                       // largest K of the per-(sub-range, column half, user) candidate lists
+constexpr int EV_MAX_K = 256;                       // largest K of the tensor path: "long lists" are EV_LIST_K < K <= EV_MAX_K
+constexpr int EV_POOL_PER_K = 8;                    // long lists: candidate slots per user, in multiples of K
 // Every fp32 value x is split into two bf16 terms, hi = bf16(x) and lo = bf16(x - hi), so |x - hi - lo| <= 2^-16 |x|,
 // and the tensor cores accumulate  hi.lo + lo.hi + hi.hi  (three K = 64 products per tile) in fp32.  Error against the
 // canonical fp32 score, relative to sum_k |u_k i_k| <= ||u||_2 ||i||_2 (Cauchy-Schwarz):
@@ -64,7 +71,7 @@ constexpr float EV_MASK_SCORE = -10e8f;             // base/graph_recommender.py
 // largest |approx - exact| / (EV_EPS_REL ||u|| max||i||) it sees into stats[3] (parts per million): tests assert < 1e6.
 constexpr float EV_EPS_REL = 1.0e-4f;
 
-enum { EV_SAMPLE = 0, EV_FILTER = 1 };
+enum { EV_SAMPLE = 0, EV_FILTER = 1, EV_FILTER_POOL = 2 };  // EV_FILTER_POOL: the FILTER pass of long lists
 
 struct EvalParams {
     const __nv_bfloat16 *Ap;  // packed test-user rows, [2 terms: hi, lo][n_test_pad / 8][8 chunks][8 rows][8]
@@ -76,7 +83,8 @@ struct EvalParams {
     float *bucket_max;   // SAMPLE out: [n_seg * sub * EV_CSPLIT][n_test_pad][EV_BUCKETS] running maxima of every sample cell
     const float *thr;    // FILTER in:  [n_test_pad] tau - 2 eps (-inf: no bound)
     float2 *cand;        // FILTER out: [sub * EV_CSPLIT][n_test_pad][cap] (approx score, item id bits): one short list per (sub-range, column half, user)
-    int32_t *cand_cnt;   // [sub * EV_CSPLIT][n_test_pad]
+                         // FILTER_POOL out: [n_test_pad][cap], one pool per user
+    int32_t *cand_cnt;   // [sub * EV_CSPLIT][n_test_pad]; FILTER_POOL: [n_test_pad] append counters (may run past cap: overflow)
     int32_t *overflow;   // [n_test_pad] flag; [n_test_pad] = count, [n_test_pad + 2 ...] = list of flagged rows
                          // ([n_test_pad + 1] = count, [2 n_test_pad + 2 ...] = rows with more than 256 candidates: eval_rescore_kernel)
     int32_t n_test, n_items, n_tiles;
@@ -431,6 +439,10 @@ __global__ void __launch_bounds__(EV_THREADS, 1) eval_scores_kernel(const EvalPa
                 if (live) thr = P.thr[row];
                 crow = P.cand + ((int64_t)part * n_pad + row) * P.cap;
             }
+            if (MODE == EV_FILTER_POOL) {
+                if (live) thr = P.thr[row];
+                crow = P.cand + row * P.cap;
+            }
 
             for (int it = 0; it < c.n_my; ++it, ++git) {
                 const int as = git & 1;
@@ -465,12 +477,33 @@ __global__ void __launch_bounds__(EV_THREADS, 1) eval_scores_kernel(const EvalPa
                                           fmaxf(__uint_as_float(v[4 * g + 2]), __uint_as_float(v[4 * g + 3])));
                         const float m = fmaxf(fmaxf(fmaxf(m4[0], m4[1]), fmaxf(m4[2], m4[3])),
                                               fmaxf(fmaxf(m4[4], m4[5]), fmaxf(m4[6], m4[7])));
-                        if (m >= thr) {
+                        if (MODE == EV_FILTER && m >= thr) {
 #pragma unroll
                             for (int g = 0; g < 8; ++g)
                                 if (m4[g] >= thr)
                                     cnt = ev_append4(__uint_as_float(v[4 * g]), __uint_as_float(v[4 * g + 1]), __uint_as_float(v[4 * g + 2]),
                                                      __uint_as_float(v[4 * g + 3]), thr, col0 + 4 * g, cnt, P.cap, crow, (mb >> (4 * g)) & 15u);
+                        }
+                        if (MODE == EV_FILTER_POOL && m >= thr) {
+                            // long lists: the chunk's hits take their slots of the user's pool with ONE atomicAdd (the lanes of a
+                            // warp issue theirs together), so a warp waits for at most one round trip per 32 columns
+                            unsigned hm = 0;
+#pragma unroll
+                            for (int j = 0; j < 32; ++j) hm |= (__uint_as_float(v[j]) >= thr ? 1u : 0u) << j;
+                            hm &= ~mb;
+                            if (hm) {
+                                const int n = __popc(hm);
+                                int slot = atomicAdd(P.cand_cnt + row, n);
+                                if (slot + n > P.cap && slot <= P.cap && atomicExch(P.overflow + row, 1) == 0)  // this append crosses the end
+                                    P.overflow[n_pad + 2 + atomicAdd(P.overflow + n_pad, 1)] = (int32_t)row;
+                                if (slot < P.cap) {
+#pragma unroll
+                                    for (int g = 0; g < 8; ++g)
+                                        if ((hm >> (4 * g)) & 15u)
+                                            slot = ev_append4(__uint_as_float(v[4 * g]), __uint_as_float(v[4 * g + 1]), __uint_as_float(v[4 * g + 2]),
+                                                              __uint_as_float(v[4 * g + 3]), thr, col0 + 4 * g, slot, P.cap, crow, (mb >> (4 * g)) & 15u);
+                                }
+                            }
                         }
                     }
                 }
@@ -540,17 +573,62 @@ __device__ __forceinline__ bool is_train_item(const int32_t *__restrict__ a, int
     }
     return lo < end && __ldg(a + lo) == v;
 }
+// Block-wide bitonic sort of n (a power of two) keys in shared memory, largest first.  The whole block calls it after a
+// __syncthreads() that publishes the keys; it returns after one that publishes the result.
+__device__ __forceinline__ void block_sort_desc(unsigned long long *a, int n) {
+    for (int k = 2; k <= n; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int p = threadIdx.x; p < n / 2; p += blockDim.x) {
+                const int i = ((p & ~(j - 1)) << 1) | (p & (j - 1));  // the lower element of the p-th pair, partner i + j
+                const unsigned long long x = a[i], y = a[i + j];
+                if ((i & k) == 0 ? x < y : x > y) {  // descending runs where bit k of i is clear
+                    a[i] = y;
+                    a[i + j] = x;
+                }
+            }
+            __syncthreads();
+        }
+    }
+}
 
 // ------------------------------------------------------------------------------------------ tau
 // One warp per test user: tau = K-th largest of the n_seg * 32 bucket maxima of the sample pass.  Every bucket
 // maximum is the score of a distinct unmasked item, so at least K items score >= tau: tau is a lower bound of
 // the user's K-th best approximate score.  Fewer than K non-empty buckets: no bound (-inf).
 // thr = tau - 2 eps with eps = EV_EPS_REL * ||u|| * max ||i|| (see EV_EPS_REL).
+// LONG (64 < K <= 256): no merging -- up to 16 keys per lane, 512 bucket maxima >= 2 K -- and the K-th largest key is built
+// bit by bit (the largest t that at least K keys reach; keys are unique, so t is one of them): 64 warp-wide counts, not K rounds.
+template <bool LONG>
 __global__ void __launch_bounds__(128) eval_tau_kernel(const float *__restrict__ bucket_max, int n_seg, int64_t n_pad, int n_test,
                                                        int K, const float *__restrict__ slack, float *__restrict__ thr) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int64_t row = (int64_t)blockIdx.x * 4 + warp;
     if (row >= n_test) return;
+    if constexpr (LONG) {
+        unsigned long long keys[16];
+#pragma unroll
+        for (int s = 0; s < 16; ++s) {
+            const float v = s < n_seg ? bucket_max[((int64_t)s * n_pad + row) * EV_BUCKETS + lane] : -CUDART_INF_F;
+            keys[s] = v > -CUDART_INF_F ? rank_key(v, s * EV_BUCKETS + lane) : 0ull;  // 0: empty bucket (or NaN), never counted
+        }
+        unsigned long long t = 0ull;
+        for (int b = 63; b >= 0; --b) {
+            const unsigned long long c = t | (1ull << b);
+            unsigned n = 0;
+#pragma unroll
+            for (int s = 0; s < 16; ++s) n += keys[s] >= c;
+            if (__reduce_add_sync(0xffffffffu, n) >= (unsigned)K) t = c;
+        }
+        if (lane == 0) {
+            float tau = -CUDART_INF_F;  // t == 0: fewer than K non-empty buckets
+            if (t != 0ull) {
+                const uint32_t ob = (uint32_t)(t >> 32);
+                tau = __uint_as_float((ob & 0x80000000u) ? (ob & 0x7fffffffu) : ~ob);
+            }
+            thr[row] = tau - slack[row];
+        }
+        return;
+    }
     // Up to 16 bucket maxima per lane are merged down to 4 (the maximum of a group of buckets is the score of one
     // item of the union bucket): 128 disjoint buckets over the whole sample, a K-th largest within 1-2 ranks of the one
     // over 512 buckets at a quarter of the selection work.
@@ -592,6 +670,28 @@ __global__ void __launch_bounds__(128) eval_tau_kernel(const float *__restrict__
 // ------------------------------------------------------------------------------------------ 3. rescore
 constexpr int RS_WARPS = 4;
 constexpr int RS_CAP = 1024;  // candidates of one user held in shared memory
+constexpr int RS_POOL_MAX = 2048;  // long lists: largest pool of one user (EV_POOL_PER_K * EV_MAX_K), sorted by one block
+constexpr int RS_POOL_WARPS = 8;
+
+// stats of one user's re-scoring: candidates, survivors, and the observed error in parts per million of the bound
+// eps = slack / 2 (must stay below 1e6)
+__device__ __forceinline__ void rs_add_stats(unsigned long long *__restrict__ stats, int n_c, int n_keep, float worst, float slack) {
+    atomicAdd(stats + 0, (unsigned long long)n_c);
+    atomicAdd(stats + 1, (unsigned long long)n_keep);
+    atomicMax(stats + 3, (unsigned long long)(worst / (0.5f * slack) * 1.0e6f));
+}
+// fewer than K unmasked items in the whole catalogue: the reference then returns masked items (-10e8) in ascending id order
+// (oracle topk_exact keeps them as candidates).  Positions filled .. K-1 of the row, thread t of `step` takes t, t + step, ...
+__device__ __forceinline__ void rs_fill_masked(const int64_t *__restrict__ train_indptr, const int32_t *__restrict__ train_indices,
+                                               int32_t u, int64_t row, int K, int filled, int t, int step, int32_t *__restrict__ out_ids,
+                                               float *__restrict__ out_scores) {
+    const int64_t t0 = train_indptr[u], t1 = train_indptr[u + 1];
+    for (int r = filled + t; r < K; r += step) {
+        const int64_t q = t0 + (r - filled);
+        out_ids[row * K + r] = q < t1 ? train_indices[q] : -1;
+        out_scores[row * K + r] = EV_MASK_SCORE;
+    }
+}
 
 // One warp per test user.  (a) the candidates' approximate scores give the approximate K-th best tau_a;
 // (b) candidates below tau_a - 2 eps cannot be in the exact top-K and are dropped; (c) the survivors are
@@ -599,15 +699,87 @@ constexpr int RS_CAP = 1024;  // candidates of one user held in shared memory
 // Two launches share the users: CAP = 256 (most users: 2 KB of keys per warp, 64 registers, 8 blocks per SM -- the kernel is a chain
 // of dependent memory round trips per warp, so resident warps are what it needs) takes the lists of up to 256 candidates and
 // lists the rows with more; the CAP = RS_CAP launch (LO >= 0) walks that list.
-template <int CAP, int LO, int MINB>
-__global__ void __launch_bounds__(RS_WARPS * 32, MINB) eval_rescore_kernel(
+// UW > 1 (long lists): one block of UW warps per user, whose pool of up to CAP candidates (the plan's cap, rounded up to a power of
+// two, of dynamic shared memory) is sorted by (a) approximate and (d) exact key with a block-wide bitonic sort: after the first sort
+// the K-th best is keys[K - 1] and the survivors of (b) are a prefix, so no step takes K dependent rounds.
+template <int CAP, int LO, int MINB, int UW = 1>
+__global__ void __launch_bounds__(UW > 1 ? UW * 32 : RS_WARPS * 32, MINB) eval_rescore_kernel(
     const float *__restrict__ user_emb, const float *__restrict__ item_emb, int D, const int32_t *__restrict__ test_users,
     const int64_t *__restrict__ train_indptr, const int32_t *__restrict__ train_indices, const float2 *__restrict__ cand,
     const int32_t *__restrict__ cand_cnt, const float *__restrict__ slack, int32_t *__restrict__ overflow, int n_parts,
     int64_t n_pad, int cap, int n_test, int K, int32_t *__restrict__ out_ids, float *__restrict__ out_scores,
     unsigned long long *__restrict__ stats) {
     __shared__ float u_sm[RS_WARPS][128];
-    __shared__ unsigned long long keys[RS_WARPS][CAP];
+    __shared__ unsigned long long keys[RS_WARPS][UW > 1 ? 1 : CAP];  // UW > 1: the keys live in dynamic shared memory
+    if constexpr (UW > 1) {
+        extern __shared__ unsigned long long pool[];
+        __shared__ int s_keep;
+        __shared__ unsigned s_worst;
+        const int64_t row = blockIdx.x;
+        if (row >= n_test || overflow[row]) return;  // overflowed pools are handled by eval_brute_kernel
+        const int n_c = min(cand_cnt[row], cap);
+        const int32_t u = test_users[row];
+        for (int k = threadIdx.x; k < D; k += UW * 32) u_sm[0][k] = user_emb[(int64_t)u * D + k];
+        int n_pow = 1;
+        while (n_pow < n_c) n_pow <<= 1;
+        // (a) approximate keys, padded with 0 (below every key) to a power of two, sorted best first
+        const float2 *lst = cand + row * cap;
+        for (int j = threadIdx.x; j < n_pow; j += UW * 32) {
+            unsigned long long k = 0ull;
+            if (j < n_c) {
+                const float2 c = lst[j];
+                k = rank_key(c.x, __float_as_int(c.y));
+            }
+            pool[j] = k;
+        }
+        if (threadIdx.x == 0) {
+            s_keep = 0;
+            s_worst = 0u;
+        }
+        __syncthreads();
+        block_sort_desc(pool, n_pow);
+        // (b) keep keys >= (tau_a - 2 eps), tau_a = the K-th best approximate score: a prefix of the sorted pool
+        unsigned long long keep_key = 0ull;
+        if (n_c >= K) {
+            const uint32_t ob = (uint32_t)(pool[K - 1] >> 32);
+            const float tau_a = __uint_as_float((ob & 0x80000000u) ? (ob & 0x7fffffffu) : ~ob);
+            keep_key = (unsigned long long)orderable(tau_a - slack[row]) << 32;
+        }
+        for (int j = threadIdx.x; j < n_c; j += UW * 32)
+            if (pool[j] >= keep_key && (j + 1 == n_c || pool[j + 1] < keep_key)) s_keep = j + 1;
+        __syncthreads();
+        const int n_keep = s_keep;
+        // (c) exact re-scoring in place; the slots up to the next power of two are cleared for the second sort
+        int n_pow2 = 1;
+        while (n_pow2 < n_keep) n_pow2 <<= 1;
+        float worst = 0.f;
+        for (int j = threadIdx.x; j < n_pow2; j += UW * 32) {
+            unsigned long long nk = 0ull;
+            if (j < n_keep) {
+                const unsigned long long k = pool[j];
+                const int id = (int32_t)(0xffffffffu - (uint32_t)(k & 0xffffffffu));
+                const float ex = exact_score(u_sm[0], item_emb + (int64_t)id * D, D);
+                const uint32_t ob = (uint32_t)(k >> 32);
+                worst = fmaxf(worst, fabsf(__uint_as_float((ob & 0x80000000u) ? (ob & 0x7fffffffu) : ~ob) - ex));
+                nk = rank_key(ex, id);
+            }
+            pool[j] = nk;
+        }
+        if (worst > 0.f) atomicMax(&s_worst, __float_as_uint(worst));  // worst >= 0: bit order = value order
+        __syncthreads();
+        // (d) exact top-K
+        block_sort_desc(pool, n_pow2);
+        const int filled = n_keep < K ? n_keep : K;
+        for (int r = threadIdx.x; r < filled; r += UW * 32) {
+            const unsigned long long k = pool[r];
+            const uint32_t ob = (uint32_t)(k >> 32);
+            out_ids[row * K + r] = (int32_t)(0xffffffffu - (uint32_t)(k & 0xffffffffu));
+            out_scores[row * K + r] = __uint_as_float((ob & 0x80000000u) ? (ob & 0x7fffffffu) : ~ob);
+        }
+        if (threadIdx.x == 0 && stats) rs_add_stats(stats, n_c, n_keep, __uint_as_float(s_worst), slack[row]);
+        rs_fill_masked(train_indptr, train_indices, u, row, K, filled, threadIdx.x, UW * 32, out_ids, out_scores);
+        return;
+    }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     int64_t row = (int64_t)blockIdx.x * RS_WARPS + warp;
     if (LO >= 0) {  // second launch: the rows the first one listed (one block per RS_WARPS of them; the rest of the grid leaves)
@@ -734,12 +906,7 @@ __global__ void __launch_bounds__(RS_WARPS * 32, MINB) eval_rescore_kernel(
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) worst = fmaxf(worst, __shfl_xor_sync(0xffffffffu, worst, o));
-    if (lane == 0 && stats) {
-        atomicAdd(stats + 0, (unsigned long long)n_c);
-        atomicAdd(stats + 1, (unsigned long long)n_keep);
-        // observed error in parts per million of the bound eps = slack / 2 (must stay below 1e6)
-        atomicMax(stats + 3, (unsigned long long)(worst / (0.5f * slack[row]) * 1.0e6f));
-    }
+    if (lane == 0 && stats) rs_add_stats(stats, n_c, n_keep, worst, slack[row]);
     // (d) exact top-K.  Few survivors (the usual case): the rank of a key = the number of keys that beat it = its
     // position in the list; otherwise K rounds of "best key strictly below the previous winner".
     int filled = 0;
@@ -783,14 +950,7 @@ __global__ void __launch_bounds__(RS_WARPS * 32, MINB) eval_rescore_kernel(
             ++filled;
         }
     }
-    // fewer than K unmasked items in the whole catalogue: the reference then returns masked items
-    // (-10e8) in ascending id order (oracle topk_exact keeps them as candidates)
-    const int64_t t0 = train_indptr[u], t1 = train_indptr[u + 1];
-    for (int r = filled + lane; r < K; r += 32) {
-        const int64_t q = t0 + (r - filled);
-        out_ids[row * K + r] = q < t1 ? train_indices[q] : -1;
-        out_scores[row * K + r] = EV_MASK_SCORE;
-    }
+    rs_fill_masked(train_indptr, train_indices, u, row, K, filled, lane, 32, out_ids, out_scores);
 }
 
 // ------------------------------------------------------------------------------------------ 4. brute force
@@ -862,32 +1022,37 @@ __global__ void __launch_bounds__(BF_THREADS) eval_brute_kernel(const float *__r
 // find_k_largest (util/algorithm.py:143-173) seeds its list with candidates[0:K] sorted by score and then
 // visits EVERY candidate again, including those first K (SURVEY.md F9).  Its result is the first K entries
 // of the stable merge of  A = items 0..K-1 sorted (score desc, id asc)  and  B = the exact top-K,
-// with A's entries first on equal scores.  One warp per user; K <= 64.
-__global__ void __launch_bounds__(128) eval_refquirk_kernel(const float *__restrict__ user_emb,
-                                                            const float *__restrict__ item_emb, int D,
-                                                            const int32_t *__restrict__ test_users,
-                                                            const int64_t *__restrict__ train_indptr,
-                                                            const int32_t *__restrict__ train_indices, int n_test, int K,
-                                                            int32_t *__restrict__ out_ids, float *__restrict__ out_scores) {
-    __shared__ float u_sm[4][128];
-    __shared__ float a_s[4][64], b_s[4][64];
-    __shared__ int b_id[4][64];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t row = (int64_t)blockIdx.x * 4 + warp;
+// with A's entries first on equal scores.  A group of TPU threads per user, UPB users per block, K <= KMAX: one warp per
+// user for K <= 64, one block per user for long lists.
+template <int KMAX, int UPB, int TPU>
+__global__ void __launch_bounds__(UPB * TPU) eval_refquirk_kernel(const float *__restrict__ user_emb,
+                                                                  const float *__restrict__ item_emb, int D,
+                                                                  const int32_t *__restrict__ test_users,
+                                                                  const int64_t *__restrict__ train_indptr,
+                                                                  const int32_t *__restrict__ train_indices, int n_test, int K,
+                                                                  int32_t *__restrict__ out_ids, float *__restrict__ out_scores) {
+    static_assert(TPU == 32 || UPB == 1, "a user's group is a warp or the whole block");
+    __shared__ float u_sm[UPB][128];
+    __shared__ float a_s[UPB][KMAX], b_s[UPB][KMAX];
+    __shared__ int b_id[UPB][KMAX];
+    const int warp = threadIdx.x / TPU, lane = threadIdx.x % TPU;  // warp = the user's group, lane = thread within it
+    const int64_t row = (int64_t)blockIdx.x * UPB + warp;
     if (row >= n_test) return;
     const int32_t u = test_users[row];
-    for (int k = lane; k < D; k += 32) u_sm[warp][k] = user_emb[(int64_t)u * D + k];
-    __syncwarp();
+    for (int k = lane; k < D; k += TPU) u_sm[warp][k] = user_emb[(int64_t)u * D + k];
+    if (TPU == 32) __syncwarp();
+    else __syncthreads();
     const int64_t t0 = train_indptr[u], t1 = train_indptr[u + 1];
-    for (int j = lane; j < K; j += 32) {
+    for (int j = lane; j < K; j += TPU) {
         float s = exact_score(u_sm[warp], item_emb + (int64_t)j * D, D);
         if (is_train_item(train_indices, t0, t1, j)) s = EV_MASK_SCORE;
         a_s[warp][j] = s;
         b_s[warp][j] = out_scores[row * K + j];
         b_id[warp][j] = out_ids[row * K + j];
     }
-    __syncwarp();
-    for (int j = lane; j < K; j += 32) {
+    if (TPU == 32) __syncwarp();
+    else __syncthreads();
+    for (int j = lane; j < K; j += TPU) {
         // position of A_j in the merge: A entries ahead of it + B entries with a strictly larger score
         const float s = a_s[warp][j];
         int pos = 0;
@@ -916,9 +1081,11 @@ struct EvalPlan {
     int64_t n_test_pad, n_items_pad;
     int n_tiles, cap, n_brute_blocks, n_mblk;
     int n_seg, seg_tiles, seg_pitch, s_sub, s_sub_tiles;  // sample pass: segment y scores tiles [y * seg_pitch, + seg_tiles) in s_sub sub-ranges
+    int stride;                                           // the sample pass scores 1 / stride of the catalogue
     int f_sub, f_sub_tiles;                               // filter pass: all tiles in f_sub sub-ranges
     size_t off_ap, off_bp, off_slack, off_maxnorm, off_bucket, bucket_bytes, off_thr, off_cand, off_cnt, off_overflow, off_scratch, total;
     bool tensor;
+    bool pool;  // long lists (EV_LIST_K < K <= EV_MAX_K): one candidate pool of `cap` slots per user
 };
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
@@ -929,7 +1096,8 @@ constexpr int EV_CELLS_PER_SM = 16;      // cells per CTA of the persistent grid
 static EvalPlan make_plan(int64_t n_test, int64_t n_items, int D, int K, int engine) {
     EvalPlan p;
     memset(&p, 0, sizeof(p));
-    p.tensor = engine != 1 && D == EV_D && K <= 64 && n_test > 0;
+    p.tensor = engine != 1 && D == EV_D && K <= EV_MAX_K && n_test > 0;
+    p.pool = p.tensor && K > EV_LIST_K;
     p.n_test_pad = ceil_div(n_test > 0 ? n_test : 1, EV_BM) * EV_BM;
     p.n_items_pad = ceil_div(n_items > 0 ? n_items : 1, EV_BN) * EV_BN;
     p.n_tiles = (int)(p.n_items_pad / EV_BN);
@@ -953,22 +1121,40 @@ static EvalPlan make_plan(int64_t n_test, int64_t n_items, int D, int K, int eng
         int cap = (4 * K + 7) / 8 * 8;
         if (cap < 64) cap = 64;
         if (cap > 512) cap = 512;
+        // long lists: slots scale with the users, not with the lists.  A user keeps ~4.5 - 5.5 K candidates (K-th of 2 K bucket
+        // maxima from the 1 / 4 sample), so its pool holds EV_POOL_PER_K * K; at most the f_sub * 2 * 256 slots a user owns at
+        // K = 64, so that no long list needs more workspace than K = 64 at the same shape.  8 K <= 2048 keys: one block of
+        // eval_rescore_kernel sorts the whole pool in 16 KB of shared memory.
+        if (p.pool) {
+            cap = EV_POOL_PER_K * K;
+            if (cap > p.f_sub * EV_CSPLIT * 256) cap = p.f_sub * EV_CSPLIT * 256;
+        }
         p.cap = cap;
     }
-    // sample pass: n_seg contiguous segments spread evenly over the catalogue, together 1 / EV_SAMPLE_STRIDE of it;
+    // sample pass: n_seg contiguous segments spread evenly over the catalogue, together 1 / stride of it;
     // at least 4 segments (128 buckets >= K), each cut into sub-ranges of at least 4 tiles for the scheduler
     int seg = (int)ceil_div(2 * EV_PLAN_SMS, p.n_mblk);
     if (seg < 4) seg = 4;
     if (seg > 8) seg = 8;  // eval_tau_kernel holds n_seg * sub * EV_CSPLIT <= 16 keys per lane
+    // long lists: 8 segments of one sub-range each, so all 16 sets of 32 buckets exist (512 bucket maxima >= 2 K) whatever the
+    // number of users (5 - 7 segments would leave 10 - 14 sets); the same number of cells as 4 segments of 2 sub-ranges
+    if (p.pool) seg = 8;
     if (seg > p.n_tiles) seg = p.n_tiles;
     p.seg_pitch = p.n_tiles / seg;
     p.n_seg = seg;
-    p.seg_tiles = (int)ceil_div(p.seg_pitch, EV_SAMPLE_STRIDE);
+    // long lists whose pool is capped below 8 K (many users: few sub-ranges) sample a larger share.  With N = 512 bucket maxima a
+    // user keeps about -N ln(1 - K / N) * stride <= 1.39 K * stride candidates (N >= 2 K), and a pool that fills up costs the
+    // brute-force kernel.  A catalogue of fewer than 8 tiles has fewer sets, but then seg_pitch = 1 and the sample is all of it.
+    p.stride = EV_SAMPLE_STRIDE;
+    if (p.pool)
+        while (p.stride > 1 && p.cap < 2 * K * p.stride) p.stride /= 2;
+    p.seg_tiles = (int)ceil_div(p.seg_pitch, p.stride);
     {
         int64_t sub = ceil_div(want_ranges, seg);
         const int64_t max_sub = p.seg_tiles / 4 > 0 ? p.seg_tiles / 4 : 1;
         if (sub > max_sub) sub = max_sub;
         if (sub > 8 / seg) sub = 8 / seg;  // every (segment, sub-range, column half) owns 32 buckets; eval_tau_kernel merges <= 16 sets
+        if (p.pool) sub = 1;  // long lists: 8 segments x 1 sub-range x 2 column halves = 16 sets
         if (sub < 1) sub = 1;
         p.s_sub_tiles = (int)ceil_div(p.seg_tiles, sub);
         p.s_sub = (int)ceil_div(p.seg_tiles, p.s_sub_tiles);
@@ -984,8 +1170,9 @@ static EvalPlan make_plan(int64_t n_test, int64_t n_items, int D, int K, int eng
         p.bucket_bytes = (size_t)8 * EV_CSPLIT * p.n_test_pad * EV_BUCKETS * 4;
         p.off_bucket = o; o = align_up(o + p.bucket_bytes, 256);
         p.off_thr = o; o = align_up(o + (size_t)p.n_test_pad * 4, 256);
-        p.off_cand = o; o = align_up(o + (size_t)p.f_sub * EV_CSPLIT * p.n_test_pad * p.cap * 8, 256);
-        p.off_cnt = o; o = align_up(o + (size_t)p.f_sub * EV_CSPLIT * p.n_test_pad * 4, 256);
+        const size_t lists = p.pool ? (size_t)p.n_test_pad : (size_t)p.f_sub * EV_CSPLIT * p.n_test_pad;
+        p.off_cand = o; o = align_up(o + lists * p.cap * 8, 256);
+        p.off_cnt = o; o = align_up(o + lists * 4, 256);
     }
     p.off_overflow = o; o = align_up(o + (size_t)(3 * p.n_test_pad + 2) * 4, 256);
     p.off_scratch = o; o = align_up(o + (size_t)p.n_brute_blocks * (size_t)(n_items > 0 ? n_items : 1) * 4, 256);
@@ -1039,13 +1226,13 @@ int hgr_fullrank_topk_f32(const float *user_emb, int64_t n_users, const float *i
     HGR_REQUIRE(K >= 1 && K <= n_items, "K = %d must be in [1, n_items = %lld]", K, (long long)n_items);
     HGR_REQUIRE(mode == 0 || mode == 1, "mode %d unknown (0 exact, 1 refquirk)", mode);
     HGR_REQUIRE(engine >= 0 && engine <= 2, "engine %d unknown (0 auto, 1 simt, 2 tensor)", engine);
-    HGR_REQUIRE(mode == 0 || K <= 64, "refquirk mode supports K <= 64, got %d", K);
+    HGR_REQUIRE(mode == 0 || K <= EV_MAX_K, "refquirk mode supports K <= 256, got %d", K);
     HGR_REQUIRE(n_items < (int64_t)0x7fffff00 && n_test < (int64_t)0x7fffff00, "dimension does not fit int32");
     if (n_test == 0) return HGR_OK;
     HGR_REQUIRE(user_emb && item_emb && test_users && train_indptr && out_ids && out_scores, "NULL argument");
     HGR_REQUIRE(aligned16(user_emb) && aligned16(item_emb), "embedding tables must be 16-byte aligned");
     const EvalPlan p = make_plan(n_test, n_items, D, K, engine);
-    HGR_REQUIRE(engine != 2 || p.tensor, "tensor engine needs D == 64 and K <= 64");
+    HGR_REQUIRE(engine != 2 || p.tensor, "tensor engine needs D == 64 and K <= 256");
     if (workspace == nullptr || workspace_bytes < p.total)
         return set_error(HGR_ERR_WORKSPACE, "fullrank_topk workspace: need %zu bytes, got %zu", p.total, workspace_bytes);
     HGR_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "workspace must be 256-byte aligned");
@@ -1092,8 +1279,9 @@ int hgr_fullrank_topk_f32(const float *user_emb, int64_t n_users, const float *i
         P.cap = p.cap;
         const size_t smem = 1024 + (size_t)EvalSmem::END;
         HGR_CUDA_OK(ensure_scores_smem<EV_SAMPLE>(smem));
-        HGR_CUDA_OK(ensure_scores_smem<EV_FILTER>(smem));
-        HGR_CUDA_OK(cudaMemsetAsync(P.cand_cnt, 0, (size_t)p.f_sub * EV_CSPLIT * p.n_test_pad * 4, st));  // dead rows and empty cells write nothing
+        HGR_CUDA_OK(p.pool ? ensure_scores_smem<EV_FILTER_POOL>(smem) : ensure_scores_smem<EV_FILTER>(smem));
+        // dead rows and empty cells write nothing; the pools' append counters start at 0
+        HGR_CUDA_OK(cudaMemsetAsync(P.cand_cnt, 0, (p.pool ? (size_t)1 : (size_t)p.f_sub * EV_CSPLIT) * p.n_test_pad * 4, st));
         const int n_sm = device_sm_count();
         // persistent grids: one CTA per SM walks its share of the cells (EvalParams)
         P.n_seg = p.n_seg;
@@ -1104,7 +1292,10 @@ int hgr_fullrank_topk_f32(const float *user_emb, int64_t n_users, const float *i
         int64_t cells = (int64_t)p.n_mblk * P.n_seg * P.sub;
         eval_scores_kernel<EV_SAMPLE><<<(unsigned)(cells < n_sm ? cells : n_sm), EV_THREADS, smem, st>>>(P);
         HGR_LAUNCH_OK("eval_scores_kernel<sample>");
-        eval_tau_kernel<<<(unsigned)ceil_div(n_test, 4), 128, 0, st>>>(P.bucket_max, p.n_seg * p.s_sub * EV_CSPLIT, p.n_test_pad, (int)n_test, K, slack, thr);
+        if (p.pool)
+            eval_tau_kernel<true><<<(unsigned)ceil_div(n_test, 4), 128, 0, st>>>(P.bucket_max, p.n_seg * p.s_sub * EV_CSPLIT, p.n_test_pad, (int)n_test, K, slack, thr);
+        else
+            eval_tau_kernel<false><<<(unsigned)ceil_div(n_test, 4), 128, 0, st>>>(P.bucket_max, p.n_seg * p.s_sub * EV_CSPLIT, p.n_test_pad, (int)n_test, K, slack, thr);
         HGR_LAUNCH_OK("eval_tau_kernel");
         P.n_seg = 1;
         P.seg_pitch = 0;
@@ -1112,25 +1303,40 @@ int hgr_fullrank_topk_f32(const float *user_emb, int64_t n_users, const float *i
         P.sub = p.f_sub;
         P.sub_tiles = p.f_sub_tiles;
         cells = (int64_t)p.n_mblk * P.sub;
-        eval_scores_kernel<EV_FILTER><<<(unsigned)(cells < n_sm ? cells : n_sm), EV_THREADS, smem, st>>>(P);
-        HGR_LAUNCH_OK("eval_scores_kernel<filter>");
-        eval_rescore_kernel<256, -1, 8><<<(unsigned)ceil_div(n_test, RS_WARPS), RS_WARPS * 32, 0, st>>>(
-            user_emb, item_emb, D, test_users, train_indptr, train_indices, P.cand, P.cand_cnt, slack, overflow,
-            p.f_sub * EV_CSPLIT, p.n_test_pad, p.cap, (int)n_test, K, out_ids, out_scores, st64);
-        HGR_LAUNCH_OK("eval_rescore_kernel<256>");
-        eval_rescore_kernel<RS_CAP, 256, 1><<<(unsigned)ceil_div(n_test, RS_WARPS), RS_WARPS * 32, 0, st>>>(
-            user_emb, item_emb, D, test_users, train_indptr, train_indices, P.cand, P.cand_cnt, slack, overflow,
-            p.f_sub * EV_CSPLIT, p.n_test_pad, p.cap, (int)n_test, K, out_ids, out_scores, st64);
-        HGR_LAUNCH_OK("eval_rescore_kernel<1024>");
+        if (p.pool) {
+            eval_scores_kernel<EV_FILTER_POOL><<<(unsigned)(cells < n_sm ? cells : n_sm), EV_THREADS, smem, st>>>(P);
+            HGR_LAUNCH_OK("eval_scores_kernel<filter_pool>");
+            int pool_pow = 1;
+            while (pool_pow < p.cap) pool_pow <<= 1;
+            eval_rescore_kernel<RS_POOL_MAX, -1, 4, RS_POOL_WARPS><<<(unsigned)n_test, RS_POOL_WARPS * 32, (size_t)pool_pow * 8, st>>>(
+                user_emb, item_emb, D, test_users, train_indptr, train_indices, P.cand, P.cand_cnt, slack, overflow, 1,
+                p.n_test_pad, p.cap, (int)n_test, K, out_ids, out_scores, st64);
+            HGR_LAUNCH_OK("eval_rescore_kernel<pool>");
+        } else {
+            eval_scores_kernel<EV_FILTER><<<(unsigned)(cells < n_sm ? cells : n_sm), EV_THREADS, smem, st>>>(P);
+            HGR_LAUNCH_OK("eval_scores_kernel<filter>");
+            eval_rescore_kernel<256, -1, 8><<<(unsigned)ceil_div(n_test, RS_WARPS), RS_WARPS * 32, 0, st>>>(
+                user_emb, item_emb, D, test_users, train_indptr, train_indices, P.cand, P.cand_cnt, slack, overflow,
+                p.f_sub * EV_CSPLIT, p.n_test_pad, p.cap, (int)n_test, K, out_ids, out_scores, st64);
+            HGR_LAUNCH_OK("eval_rescore_kernel<256>");
+            eval_rescore_kernel<RS_CAP, 256, 1><<<(unsigned)ceil_div(n_test, RS_WARPS), RS_WARPS * 32, 0, st>>>(
+                user_emb, item_emb, D, test_users, train_indptr, train_indices, P.cand, P.cand_cnt, slack, overflow,
+                p.f_sub * EV_CSPLIT, p.n_test_pad, p.cap, (int)n_test, K, out_ids, out_scores, st64);
+            HGR_LAUNCH_OK("eval_rescore_kernel<1024>");
+        }
     }
     eval_brute_kernel<<<(unsigned)p.n_brute_blocks, BF_THREADS, 0, st>>>(user_emb, item_emb, D, (int)n_items, test_users,
                                                                         train_indptr, train_indices, overflow, p.tensor ? 1 : 0,
                                                                         p.n_test_pad, (int)n_test, K, scratch, out_ids, out_scores, st64);
     HGR_LAUNCH_OK("eval_brute_kernel");
-    if (mode == 1) {
-        eval_refquirk_kernel<<<(unsigned)ceil_div(n_test, 4), 128, 0, st>>>(user_emb, item_emb, D, test_users, train_indptr,
-                                                                           train_indices, (int)n_test, K, out_ids, out_scores);
+    if (mode == 1 && K <= EV_LIST_K) {
+        eval_refquirk_kernel<EV_LIST_K, 4, 32><<<(unsigned)ceil_div(n_test, 4), 128, 0, st>>>(user_emb, item_emb, D, test_users, train_indptr,
+                                                                                              train_indices, (int)n_test, K, out_ids, out_scores);
         HGR_LAUNCH_OK("eval_refquirk_kernel");
+    } else if (mode == 1) {
+        eval_refquirk_kernel<EV_MAX_K, 1, EV_MAX_K><<<(unsigned)n_test, EV_MAX_K, 0, st>>>(user_emb, item_emb, D, test_users, train_indptr,
+                                                                                           train_indices, (int)n_test, K, out_ids, out_scores);
+        HGR_LAUNCH_OK("eval_refquirk_kernel<long>");
     }
     return HGR_OK;
 }

@@ -647,7 +647,8 @@ def fullrank_topk_sharded(g: DistGraph, out_u: torch.Tensor, out_i: torch.Tensor
     """Full-ranking evaluation sharded by user (SURVEY.md 8e): every rank ranks ITS users (``test_users_local`` index the
     rank's own user rows ``out_u``; ``train_indptr_own / train_indices_own`` is the training matrix of those rows with GLOBAL
     item ids) against the whole item table, which is assembled once from the gathered rows.  Returns this rank's
-    ``(ids, scores[, stats])`` with global item ids; recommendation lists never cross ranks (metric sums do, as scalars)."""
+    ``(ids, scores[, stats])`` with global item ids; recommendation lists never cross ranks (metric sums do, as scalars).
+    ``k`` and ``mode`` have the range of ``evaluation.fullrank_topk`` (up to 256 in both modes)."""
     from . import evaluation
 
     with torch.no_grad():

@@ -35,7 +35,8 @@ def fullrank_topk(user_emb: torch.Tensor, item_emb: torch.Tensor, test_users: to
                   train_indices: torch.Tensor, k: int, mode: str = "exact", engine: str = "auto", return_stats: bool = False):
     """Top-``k`` items for every test user.  Returns device tensors ``(ids int32 [n_test, k], scores float32
     [n_test, k])`` (+ a uint64[4] stats tensor).  ``train_indptr`` (int64 [n_users + 1]) / ``train_indices``
-    (int32, ascending inside a row) are the training interaction matrix used as the mask."""
+    (int32, ascending inside a row) are the training interaction matrix used as the mask.  ``k`` goes to the C ABI unchanged:
+    both modes take ``k <= 256`` (the tensor-core path when the width is 64), ``mode='exact'`` also any larger ``k`` (SIMT path)."""
     if not (user_emb.is_cuda and item_emb.is_cuda):
         raise _lib.HgrError("embedding tables must be CUDA tensors (no CPU path)")
     if user_emb.dtype != torch.float32 or item_emb.dtype != torch.float32 or user_emb.dim() != 2 or item_emb.dim() != 2:
@@ -129,7 +130,8 @@ class EvalData:
 def test(recommender, user_emb: torch.Tensor, item_emb: torch.Tensor, mode: str = "refquirk", engine: str = "auto"):
     """Drop-in body for ``GraphRecommender.test``: ``rec_list[raw_user] = [(raw_item, score), ...]`` of length
     ``recommender.max_N`` for every user of ``recommender.data.test_set``.  ``mode='refquirk'`` (default here)
-    reproduces the reference's lists exactly; ``'exact'`` gives the duplicate-free top-K."""
+    reproduces the reference's lists exactly; ``'exact'`` gives the duplicate-free top-K.  ``max_N`` up to 256 works in both
+    modes (``fullrank_topk``)."""
     ev = getattr(recommender, "_hgr_eval_data", None)
     if ev is None:
         ev = EvalData(recommender.data, device=user_emb.device)

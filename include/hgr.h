@@ -319,11 +319,12 @@ int hgr_bpr_l2_bwd_owned_f32(const float *table, int64_t n_rows, int32_t D, cons
  * summation order is unspecified); out_scores holds exactly those values.
  * mode 0 ("exact"):    true top-K, score descending, ties by ascending item id, no duplicates.
  * mode 1 ("refquirk"): find_k_largest as shipped, which visits the first K candidates twice, so an item
- *                      with id < K that makes the list appears twice (SURVEY.md F9); K <= 64.
- * engine 0: tcgen05 tensor path when D == 64 and K <= 64 (candidate generation with 2 x bf16 split operands
+ *                      with id < K that makes the list appears twice (SURVEY.md F9); K <= 256.
+ * engine 0: tcgen05 tensor path when D == 64 and K <= 256 (candidate generation with 2 x bf16 split operands
  *           and a proven error bound, exact fp32 re-scoring of the candidates; results identical to
  *           engine 1), else SIMT.
- * engine 1: SIMT fp32 brute force.   engine 2: tensor path or HGR_ERR_INVALID.
+ * engine 1: SIMT fp32 brute force (any K <= n_items in mode 0).
+ * engine 2: tensor path (D == 64 and K <= 256) or HGR_ERR_INVALID.
  * stats (device uint64[4], optional, caller zeroes): candidates emitted by the tensor stage, candidates
  * re-scored, users that overflowed to the brute-force fallback, and the largest observed
  * |tensor score - fp32 score| in parts per million of the proven error bound (always < 1e6).
