@@ -14,7 +14,8 @@
 //   ssl_finish_kernel    per-row loss terms -> mean (single block, fixed order), per-row backward coefficients
 //   ssl_pass_kernel<1/2> backward, logits recomputed tile by tile (flash-style): dA_j = c_j/(M T) (sum_k w_jk b_k - b_j),
 //                        dB_k = 1/(M T) (sum_j c_j w_jk a_j - c_k a_k), w_jk = exp(l_jk) / deno_j; then the
-//                        normalisation backward and the scatter to the table rows (nodes are unique: plain stores).
+//                        normalisation backward and the scatter to the table rows (atomic adds: a repeated id gets the
+//                        sum of its gradients).
 #include <math_constants.h>
 
 #include "hgr_internal.cuh"

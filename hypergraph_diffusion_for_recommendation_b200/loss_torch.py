@@ -220,8 +220,9 @@ class _SslLoss(torch.autograd.Function):
 
 
 def contrastLoss(embeds1, embeds2, nodes, temp):
-    """util/loss_torch.py:103-110.  ``nodes`` must be unique (the reference passes ``torch.unique``); only the picked
-    rows are normalised and the [M, M] logits stay on chip."""
+    """util/loss_torch.py:103-110.  Only the picked rows are normalised and the [M, M] logits stay on chip.  The reference
+    passes ``torch.unique`` ids; a repeated id is evaluated as the reference expression does, as duplicate rows and
+    columns of the logits, and its table row gets the sum of the gradients of its copies."""
     return _SslLoss.apply(embeds1, embeds2, nodes, temp, 0, 1)
 
 

@@ -341,7 +341,8 @@ int hgr_fullrank_topk_f32(const float *user_emb, int64_t n_users, const float *i
  *   kind 0  contrastLoss(embeds1, embeds2, nodes, temp)   util/loss_torch.py:103-110 (HCCF.py:62-66, HGNN_HD3.py:345-350)
  *   kind 1  InfoNCE(view1, view2, temperature, b_cos)     util/loss_torch.py:32-40   (SGL.py:167-180)
  * E1 [n_rows1, D], E2 [n_rows2, D]; nodes int64 [M] picks the rows (NULL: rows 0..M-1 of both tables, the InfoNCE
- * call shape).  nodes must be unique (the reference passes torch.unique(...)).  normalize = F.normalize of the rows
+ * call shape).  A repeated id gives duplicate rows and columns of the logits, and its table row receives the sum of
+ * the gradients of its copies (the reference passes torch.unique(...)).  normalize = F.normalize of the rows
  * (always on for kind 0, b_cos for kind 1).  loss: device float[1].  `saved` (hgr_ssl_workspace_bytes(M, D), 256-byte
  * aligned) carries the normalised rows, row sums and coefficients to the backward call.  The [M, M] logits are never
  * materialised.  Backward: dE1 / dE2 ([n_rows, D], zero-filled by the caller; either may be NULL for a detached
